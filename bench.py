@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the matching hot path (BASELINE.json): reads/s and text Gbp/s.
 
-    python bench.py --gpus N --steps K --warmup W [--workload c3|c2|c1|tiny] [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--workload c3|c2|c1|tiny] [--impl reference] [--dump-outputs DIR]
 
 A step = one pass of the hot path over the synthetic workload: read packing + read-side signature
 index build (K1+K2), text scan with probe/verify (K3), result reduction (and, for N>1, the one
@@ -335,8 +335,8 @@ def run_reference_arm(args, wl):
             vals.append(last)
     v = statistics.mean(x["value"] for x in vals)
     full_s = statistics.mean(x["extrapolated_full_s"] for x in vals)
-    line = {"impl": "reference", "metric": "matching-path reads/s", "value": v, "unit": "reads/s", "n_gpus": args.gpus, "steps": args.steps,
-            "warmup": args.warmup, "ms_per_step": full_s * 1e3, "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
+    line = {"impl": "reference", "metric": "matching-path reads/s", "value": v, "unit": "reads/s", "n_gpus": args.gpus, "steps": n_timed,
+            "warmup": n_warm, "ms_per_step": full_s * 1e3, "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
             "dtype": "u64", "data": "synthetic", "config": workload_config(wl),
             "executions": {"warmup": n_warm, "timed": n_timed, "note": "the sample is run from scratch each time; more repetitions would only repeat it"},
             "text_gbp_per_s": wl["n"] / full_s / 1e9,
@@ -365,6 +365,48 @@ def kernel_table(workload: str, world: int, as_rank: str):
 # scattered loads served by L2: one distinct 128-byte line per cycle and SM through the L1TEX tag stage -- 277-281 G lines/s on
 # this pool's B200 for resident sets up to ~96 MB (tools/l2_resident_bench.cu, profiles/r01_l2_resident_bench.txt)
 L1TEX_LINES_PER_S = 280e9
+
+
+DUMP_READS = 1 << 19          # --dump-outputs: reads of the fixed sample whose results are written
+DUMP_BYTES = 60 << 20         # --dump-outputs: at most this many bytes of array data in all (below 64 MB with the file headers)
+
+
+def dump_outputs(out_dir: str, h, R: int, unique: bool, gaps: bool) -> dict:
+    """--dump-outputs: what the last timed step computed, as the caller of the matching path receives it, for the reads of a
+    fixed seeded sample (the same for every run of a workload), so that two builds can be compared output for output.
+    One field per file DIR/<name>.npy; integers as float64 (exact below 2^53), scores as float32.
+    matchUnique: the UniqueMatchInfo fields of each sampled read (unique_*), the score with scores, the GapInfo rows of the
+    sampled reads after the gapped pass (gaps_*).  matchAll: the real_gpu_hit16 rows the last step received for the sampled
+    reads (hits_*), in the library's order, cut to the byte budget."""
+    import numpy as np
+    from real_b200 import matcher
+    reads = np.sort(np.random.default_rng(SEED).choice(R, size=min(R, DUMP_READS), replace=False))
+    f64 = lambda a: np.asarray(a).astype(np.float64)
+    out = {}
+    if unique:
+        info, sc = h.get_unique()
+        info = info[reads]
+        out.update(unique_read=f64(reads), unique_state=f64(matcher.umi_state(info)), unique_pos=f64(matcher.umi_pos(info)),
+                   unique_file=f64(matcher.umi_file(info)), unique_err=f64(matcher.umi_err(info)), unique_frag=f64(matcher.umi_frag(info)))
+        if sc is not None:
+            out["unique_score"] = sc[reads].astype(np.float32)
+        if gaps:
+            g = h.get_gaps()
+            g = g[(g["present"] == 1) & np.isin(g["patid"], reads)]
+            out.update({"gaps_" + k: f64(g[k]) for k in ("patid", "mingap", "where", "start", "gap_pos")})
+    else:
+        rows = h.last_rows_packed()
+        rows = rows[np.isin(rows["patid"], reads)]
+        fields = ("patid", "pos", "frag", "k", "inverted")         # a real_gpu_hit16 row has no file: the one the call matched against
+        rows = rows[:DUMP_BYTES // (8 * len(fields) + 4)]
+        out.update({"hits_" + k: f64(rows[k]) for k in fields})
+        out["hits_score"] = np.ascontiguousarray(rows["score"]).astype(np.float32)
+    nbytes = sum(a.nbytes for a in out.values())
+    assert nbytes <= DUMP_BYTES, nbytes
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return {"dir": out_dir, "sampled_reads": int(reads.size), "files": len(out), "bytes": int(nbytes)}
 
 
 def ingest_probe(torch, rlib, peak_gbs: float) -> dict:
@@ -477,12 +519,20 @@ def main():
     ap.add_argument("--ref-reads", type=int, default=500_000, help="reference arm: reads of the sample")
     ap.add_argument("--cpu-text", type=int, default=16_000_000)
     ap.add_argument("--cpu-reads", type=int, default=250_000)
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="one GPU: after the timed steps, write what the last step computed to DIR/<name>.npy (the results of a fixed "
+                         "seeded sample of %d reads, at most %d MiB in all), for comparing two builds output for output"
+                         % (DUMP_READS, DUMP_BYTES >> 20))
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     wl = WORKLOADS[args.workload]
     if args.warmup < 3 and args.impl == "ours":
         print("note: fewer than 3 warm-up steps; not a reportable number", file=sys.stderr)
 
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes what the GPU path computed: not with --impl reference")
         return run_reference_arm(args, wl)
 
     import numpy as np
@@ -497,6 +547,8 @@ def main():
     local = int(os.environ.get("LOCAL_RANK", "0"))
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device: the matching path has no CPU fallback")
+    if args.dump_outputs and (world > 1 or args.as_rank):
+        raise SystemExit("--dump-outputs: one GPU running the whole job only")
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
     affinity = bind_to_gpu_numa(torch, local) if (world > 1 and not args.no_numa_bind) else {"bound": False}
@@ -647,6 +699,8 @@ def main():
     clk = clocks.stop() if rank == 0 else {}
     ms_per_step = total_ms / args.steps
     value = R / (ms_per_step * 1e-3)
+    # before anything else runs on the handle: it holds the result of the last timed step
+    dumped = dump_outputs(args.dump_outputs, h, R, unique, gaps) if args.dump_outputs else None
 
     # ---- digest of the result of the last step (outside the timed region): must not depend on the number of GPUs
     def result_digest():
@@ -834,7 +888,7 @@ def main():
                 for k in e2e_phase:
                     e2e_phase[k].append(st.get(k, 0.0))
 
-            e_steps = max(1, min(args.steps, 3))
+            e_steps = args.steps
             e_ms, _ = timed(step_host, e_steps, 1, collect_e2e)
             # the state the last end-to-end step left on the device must be the one of the device-resident steps
             e2e_digest = result_digest()
@@ -904,7 +958,7 @@ def main():
             "partition_beside_build": bool(last_stats.get("prepared_scans", 0)),
             "counts": {"windows": tot[0], "candidates": tot[1], "hits": tot[2], "seedpass": tot[3], "matchall_hits": nhits_holder[0]},
             "roofline": roofline, "cpu_baseline": cpu, "e2e": e2e, "gpu_launches": launches, "clocks": clk,
-            "device_bytes": dev_bytes, "ingest": ingest, "cpu_affinity": affinity,
+            "device_bytes": dev_bytes, "ingest": ingest, "cpu_affinity": affinity, "dump_outputs": dumped,
         }
         print(json.dumps(line), flush=True)
     if world > 1:

@@ -342,16 +342,28 @@ class Handle:
         p = C.c_void_p()
         n = C.c_uint64()
         self._check((self.L.real_gpu_match_all_packed if packed else self.L.real_gpu_match_all)(self.h, C.byref(p), C.byref(n)))
+        self._last_packed = (p.value, int(n.value)) if packed else None
         return int(n.value)
+
+    def last_rows_packed(self) -> np.ndarray:
+        """The rows the last match_all_count(packed=True) left in the library's pinned buffer, expanded like match_all_packed,
+        without matching again; valid until the handle matches again or is closed."""
+        if getattr(self, "_last_packed", None) is None:
+            raise RuntimeError("last_rows_packed: the last match call was not match_all_count(packed=True)")
+        return self._expand_hit16(*self._last_packed)
 
     def match_all_packed(self) -> np.ndarray:
         """The rows of match_all as real_gpu_hit16, expanded to the fields of HIT_DTYPE."""
         p = C.c_void_p()
         n = C.c_uint64()
         self._check(self.L.real_gpu_match_all_packed(self.h, C.byref(p), C.byref(n)))
-        out = np.zeros(n.value, dtype=HIT_DTYPE)
-        if n.value:
-            buf = (C.c_char * (n.value * HIT16_DTYPE.itemsize)).from_address(p.value)
+        return self._expand_hit16(p.value, n.value)
+
+    @staticmethod
+    def _expand_hit16(ptr: int, count: int) -> np.ndarray:
+        out = np.zeros(count, dtype=HIT_DTYPE)
+        if count:
+            buf = (C.c_char * (count * HIT16_DTYPE.itemsize)).from_address(ptr)
             r = np.frombuffer(buf, dtype=HIT16_DTYPE)
             w = r["pos_k_inv_frag"]
             out["patid"] = r["patid"]; out["pos"] = w & np.uint64((1 << 35) - 1); out["k"] = (w >> np.uint64(35)) & np.uint64(15)
