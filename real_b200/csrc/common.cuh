@@ -215,12 +215,6 @@ __host__ __device__ __forceinline__ uint32_t slot_of(uint64_t key, uint32_t keyb
 // priority -- a randomly probed 32 MB table already drops from ~278 to ~180 G probes/s, 64 MB to
 // ~105 -- while plain loads or loads carrying an evict_last policy hold ~275 G/s up to 64 MB, also with
 // a stream of touch-once data flowing through L2 at the same time.
-__device__ __forceinline__ uint64_t policy_evict_last()
-{
-        uint64_t pol;
-        asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
-        return pol;
-}
 __device__ __forceinline__ uint64_t policy_evict_normal()
 {
         uint64_t pol;

@@ -857,10 +857,10 @@ __global__ void __launch_bounds__(256, 7) k_build_sub(const uint64_t * __restric
 
 // The sub-bucket kernel of the fused build: the grouped ITEMS [sub_start[sb], sub_start[sb+1]) all carry a fragment t that
 // starts with the prefix sb, so for every table the slots of their entries lie in [sb << sub_shift, (sb+1) << sub_shift).
-// One CTA builds that piece of all three tables: item (strand, t) is an entry of table tb when t < nl[tb] (A: pairs (t,t+1),
-// B: (t,t+2), C: (t,t+3)).  The entry arrays of the three tables use the ITEM numbering: the entries of a sub-bucket sit at
+// Three CTAs build that piece of the three tables, one each: item (strand, t) is an entry of table tb when t < nl[tb] (A: pairs
+// (t,t+1), B: (t,t+2), C: (t,t+3)).  The entry arrays of the three tables use the ITEM numbering: the entries of a sub-bucket sit at
 // the front of E[tb][sub_start[sb] ...) -- no per-table offsets are needed; B and C leave the tail of each range unused.
-// Dynamic shared memory per table: presence bits and claimed bits (words u32 each) and the ranks of the words' first slots
+// Dynamic shared memory: presence bits and claimed bits (words u32 each) and the ranks of the words' first slots
 // (words u16, relative to the sub-bucket: a sub-bucket spans at most 2^16 slots).
 static const uint32_t SUB3_DUP_CAP = 256;
 struct Build3Params
@@ -872,8 +872,9 @@ struct Build3Params
         uint32_t * ndistinct[3];
 };
 
-// SPLIT: one CTA per (sub-bucket, table) -- a third of the shared memory and fewer registers per CTA, so that enough CTAs
-// are resident to hide the latencies of a kernel that is a chain of short phases (items -> presence bits -> ranks -> heads)
+// One CTA per (sub-bucket, table) -- a third of the shared memory and fewer registers per CTA than one CTA for all three
+// tables, so that enough CTAs are resident to hide the latencies of a kernel that is a chain of short phases (items -> presence
+// bits -> ranks -> heads)
 // FAST: -l 32 (fragments of 8 bases, 2^32 slots, sub-buckets of 2^16 slots): the slot of an entry relative to its sub-bucket is
 // simply the second fragment of its pair, one 16-bit field of the seed -- the general path (entry_slot) spends some twenty
 // instructions per entry and pass on runtime geometry
@@ -885,23 +886,23 @@ __device__ __forceinline__ uint32_t sub_local_slot(uint64_t seed, TableGeom cons
         return entry_slot(seed, G, t) - slot0;
 }
 
-#ifndef REAL_BUILD_MINB
-#define REAL_BUILD_MINB 6
-#endif
-template<bool SPLIT, bool FAST>
-__global__ void __launch_bounds__(256, SPLIT ? REAL_BUILD_MINB : 3) k_build_sub3(const __grid_constant__ Build3Params P)
+static const int BUILD3_MINB = 6;                               // CTAs per SM of k_build_sub3 (register bound)
+template<bool FAST>
+__global__ void __launch_bounds__(256, BUILD3_MINB) k_build_sub3(const __grid_constant__ Build3Params P)
 {
         extern __shared__ __align__(16) uint32_t sub_smem[];
         uint32_t const words = P.words;
-        constexpr int NT = SPLIT ? 1 : 3;                          // tables of this CTA
-        __shared__ SubDup dup[NT][SUB3_DUP_CAP];
-        __shared__ uint32_t ndup[NT], dist[NT];
-        uint32_t const sb = P.first_sub + (SPLIT ? blockIdx.x / 3 : blockIdx.x);
-        int const tb0 = SPLIT ? (int)(blockIdx.x % 3) : 0;
-        if ( SPLIT && ! P.G[tb0].nlists ) return;
+        __shared__ SubDup dup[SUB3_DUP_CAP];
+        __shared__ uint32_t ndup, dist;
+        uint32_t const sb = P.first_sub + blockIdx.x / 3;
+        int const tb = (int)(blockIdx.x % 3);
+        TableGeom const & G = P.G[tb];
+        if ( ! G.nlists ) return;
         uint32_t const s0 = P.sub_start[sb], s1 = P.sub_start[sb+1];
         uint32_t const slot0 = sb << P.sub_shift;
-        uint32_t const tstride = 2 * words + (words + 1) / 2;          // per table: presence bits, claimed bits (u32 each), ranks (u16, relative to s0)
+        // presence bits, claimed bits (u32 each), ranks (u16, relative to s0)
+        uint32_t * bits = sub_smem, * claimed = bits + words;
+        uint16_t * rank = reinterpret_cast<uint16_t *>(bits + 2 * words);
         // the items of the sub-bucket (some 55 KB) are pulled into L2 while the shared memory is cleared: the two passes below
         // wait for their item loads more than for anything else (a third of the stall samples), four loads per thread at a time
         for ( uint32_t i = s0 + threadIdx.x * 16; i < s1; i += 256 * 16 )
@@ -909,8 +910,8 @@ __global__ void __launch_bounds__(256, SPLIT ? REAL_BUILD_MINB : 3) k_build_sub3
                 asm volatile("prefetch.global.L2 [%0];" :: "l"(P.item_seed + i));
                 if ( ((i - s0) & 31) == 0 ) asm volatile("prefetch.global.L2 [%0];" :: "l"(P.item_val + i));
         }
-        for ( uint32_t w = threadIdx.x; w < NT * tstride; w += 256 ) sub_smem[w] = 0;
-        if ( threadIdx.x < NT ) ndup[threadIdx.x] = 0;
+        for ( uint32_t w = threadIdx.x; w < 2 * words + (words + 1) / 2; w += 256 ) sub_smem[w] = 0;
+        if ( threadIdx.x == 0 ) ndup = 0;
         __syncthreads();
         // presence bits; four items per thread and step, their loads issued together
         for ( uint32_t i0 = s0 + threadIdx.x; i0 < s1; i0 += 1024 )
@@ -928,53 +929,37 @@ __global__ void __launch_bounds__(256, SPLIT ? REAL_BUILD_MINB : 3) k_build_sub3
                         if ( i0 + (uint32_t)k * 256 < s1 )
                         {
                                 uint32_t const t = val[k] & 3;
-                                #pragma unroll
-                                for ( int u = 0; u < NT; ++u )
+                                if ( t < G.nlists )
                                 {
-                                        int const tb = tb0 + u;
-                                        if ( t < P.G[tb].nlists )
-                                        {
-                                                uint32_t const l = sub_local_slot<FAST>(seed[k], P.G[tb], t, tb, slot0);
-                                                atomicOr(&sub_smem[u * tstride + (l >> 5)], 1u << (l & 31));
-                                        }
+                                        uint32_t const l = sub_local_slot<FAST>(seed[k], G, t, tb, slot0);
+                                        atomicOr(&bits[l >> 5], 1u << (l & 31));
                                 }
                         }
         }
         __syncthreads();
-        // ranks: every thread owns a run of consecutive words of every table
-        uint32_t const wpt = (words + 255) / 256;
-        uint32_t const w0 = threadIdx.x * wpt;
-        #pragma unroll 1
-        for ( int u = 0; u < NT; ++u )
+        // ranks: every thread owns a run of consecutive words
         {
-                uint32_t * bits = sub_smem + u * tstride;
-                uint16_t * rank = reinterpret_cast<uint16_t *>(bits + 2 * words);
+                uint32_t const wpt = (words + 255) / 256;
+                uint32_t const w0 = threadIdx.x * wpt;
                 uint32_t c = 0;
                 for ( uint32_t w = w0; w < min(words, w0 + wpt); ++w ) c += __popc(bits[w]);
                 uint32_t d;
                 uint32_t run = block_excl_scan(c, &d);                    // < 2^16: a sub-bucket spans at most 2^16 slots
                 for ( uint32_t w = w0; w < min(words, w0 + wpt); ++w ) { rank[w] = (uint16_t)run; run += __popc(bits[w]); }
-                if ( threadIdx.x == 0 ) dist[u] = d;
+                if ( threadIdx.x == 0 ) dist = d;
         }
         __syncthreads();
-        #pragma unroll 1
-        for ( int u = 0; u < NT; ++u )
+        for ( uint32_t w = threadIdx.x; w < words; w += 256 )
         {
-                int const tb = tb0 + u;
-                if ( ! P.G[tb].nlists ) continue;
-                const uint32_t * bits = sub_smem + u * tstride;
-                const uint16_t * rank = reinterpret_cast<const uint16_t *>(bits + 2 * words);
-                for ( uint32_t w = threadIdx.x; w < words; w += 256 )
-                {
-                        SlotWord sw; sw.bits = bits[w]; sw.rank = s0 + rank[w];
-                        P.slots[tb][(uint64_t)sb * words + w] = sw;
-                }
-                if ( threadIdx.x == 0 && dist[u] ) atomicAdd(P.ndistinct[tb], dist[u]);
+                SlotWord sw; sw.bits = bits[w]; sw.rank = s0 + rank[w];
+                P.slots[tb][(uint64_t)sb * words + w] = sw;
         }
+        if ( threadIdx.x == 0 && dist ) atomicAdd(P.ndistinct[tb], dist);
         __syncthreads();
         // entries: the first one of a slot claims E[rank] and writes the whole 16-byte head (next = none) with one store; the
         // others (few: the tables are sparse) are set aside -- or, beyond the capacity of the list, parked in their final place
         // with the head's index in `next` -- and chained after the barrier, when every head stands
+        Entry * E = P.E[tb];
         for ( uint32_t i0 = s0 + threadIdx.x; i0 < s1; i0 += 1024 )
         {
                 uint64_t seed[4]; uint32_t val[4];
@@ -990,36 +975,28 @@ __global__ void __launch_bounds__(256, SPLIT ? REAL_BUILD_MINB : 3) k_build_sub3
                         if ( i0 + (uint32_t)k * 256 < s1 )
                         {
                                 uint32_t const t = val[k] & 3;
-                                #pragma unroll
-                                for ( int u = 0; u < NT; ++u )
+                                if ( t < G.nlists )
                                 {
-                                        int const tb = tb0 + u;
-                                        if ( t < P.G[tb].nlists )
+                                        uint32_t const l = sub_local_slot<FAST>(seed[k], G, t, tb, slot0);
+                                        uint32_t const bit = 1u << (l & 31);
+                                        uint32_t const r = s0 + rank[l >> 5] + __popc(bits[l >> 5] & (bit - 1));
+                                        if ( ! (atomicOr(&claimed[l >> 5], bit) & bit) )
                                         {
-                                                uint32_t * bits = sub_smem + u * tstride, * claimed = bits + words;
-                                                const uint16_t * rank = reinterpret_cast<const uint16_t *>(bits + 2 * words);
-                                                uint32_t const l = sub_local_slot<FAST>(seed[k], P.G[tb], t, tb, slot0);
-                                                uint32_t const bit = 1u << (l & 31);
-                                                uint32_t const r = s0 + rank[l >> 5] + __popc(bits[l >> 5] & (bit - 1));
-                                                Entry * E = P.E[tb];
-                                                if ( ! (atomicOr(&claimed[l >> 5], bit) & bit) )
+                                                Entry en; en.seed = seed[k]; en.val = val[k]; en.next = ENTRY_NONE;
+                                                *reinterpret_cast<uint4 *>(E + r) = *reinterpret_cast<const uint4 *>(&en);
+                                        }
+                                        else
+                                        {
+                                                uint32_t const j = atomicAdd(&ndup, 1u);
+                                                if ( j < SUB3_DUP_CAP )
                                                 {
-                                                        Entry en; en.seed = seed[k]; en.val = val[k]; en.next = ENTRY_NONE;
-                                                        *reinterpret_cast<uint4 *>(E + r) = *reinterpret_cast<const uint4 *>(&en);
+                                                        SubDup dd; dd.seed = seed[k]; dd.val = val[k]; dd.r = r;
+                                                        dup[j] = dd;
                                                 }
                                                 else
                                                 {
-                                                        uint32_t const j = atomicAdd(&ndup[u], 1u);
-                                                        if ( j < SUB3_DUP_CAP )
-                                                        {
-                                                                SubDup dd; dd.seed = seed[k]; dd.val = val[k]; dd.r = r;
-                                                                dup[u][j] = dd;
-                                                        }
-                                                        else
-                                                        {
-                                                                Entry en; en.seed = seed[k]; en.val = val[k]; en.next = r;
-                                                                *reinterpret_cast<uint4 *>(E + s0 + dist[u] + j) = *reinterpret_cast<const uint4 *>(&en);
-                                                        }
+                                                        Entry en; en.seed = seed[k]; en.val = val[k]; en.next = r;
+                                                        *reinterpret_cast<uint4 *>(E + s0 + dist + j) = *reinterpret_cast<const uint4 *>(&en);
                                                 }
                                         }
                                 }
@@ -1027,25 +1004,20 @@ __global__ void __launch_bounds__(256, SPLIT ? REAL_BUILD_MINB : 3) k_build_sub3
         }
         __syncthreads();
         // the set-aside entries go behind the distinct ones of this sub-bucket
-        #pragma unroll 1
-        for ( int u = 0; u < NT; ++u )
+        uint32_t const nd = min(ndup, SUB3_DUP_CAP);          // (ndup counts every same-slot entry, parked ones included)
+        for ( uint32_t j = threadIdx.x; j < nd; j += 256 )
         {
-                uint32_t const nd = min(ndup[u], SUB3_DUP_CAP);          // (ndup counts every same-slot entry, parked ones included)
-                Entry * E = P.E[tb0 + u];
-                for ( uint32_t j = threadIdx.x; j < nd; j += 256 )
-                {
-                        SubDup const dd = dup[u][j];
-                        uint32_t const o = s0 + dist[u] + j;
-                        Entry en; en.seed = dd.seed; en.val = dd.val;
-                        en.next = atomicExch(&E[dd.r].next, o);
-                        *reinterpret_cast<uint4 *>(E + o) = *reinterpret_cast<const uint4 *>(&en);
-                }
-                for ( uint32_t j = SUB3_DUP_CAP + threadIdx.x; j < ndup[u]; j += 256 )
-                {
-                        uint32_t const o = s0 + dist[u] + j;
-                        uint32_t const r = E[o].next;                        // the head's index was parked here
-                        E[o].next = atomicExch(&E[r].next, o);
-                }
+                SubDup const dd = dup[j];
+                uint32_t const o = s0 + dist + j;
+                Entry en; en.seed = dd.seed; en.val = dd.val;
+                en.next = atomicExch(&E[dd.r].next, o);
+                *reinterpret_cast<uint4 *>(E + o) = *reinterpret_cast<const uint4 *>(&en);
+        }
+        for ( uint32_t j = SUB3_DUP_CAP + threadIdx.x; j < ndup; j += 256 )
+        {
+                uint32_t const o = s0 + dist + j;
+                uint32_t const r = E[o].next;                        // the head's index was parked here
+                E[o].next = atomicExch(&E[r].next, o);
         }
 }
 

@@ -18,7 +18,6 @@
 #include <cstdlib>
 #include <cfloat>
 #include <vector>
-#include <functional>
 
 using namespace realgpu;
 
@@ -174,12 +173,8 @@ struct real_gpu
         void * stage_buf[8]; cudaStream_t stage_st[4];
 
         real_gpu_stats stats;
-        int pass_bits_override;        // REAL_GPU_PASS_BITS (tuning), -1 = automatic
-        uint64_t l2_slice_bytes;       // table bytes (presence bits + entries) one bucket may touch (REAL_GPU_L2_SLICE_MB)
-        uint64_t chunk_positions;      // text positions partitioned at a time (REAL_GPU_CHUNK_MPOS); 0 = automatic
-        int own_list_max;              // bucket shards: own buckets up to which the kept positions are listed first (REAL_GPU_OWN_LIST_MAX)
 
-        real_gpu() : n_list(0), src_packed(nullptr), src_byte_offsets(nullptr), src_packed_uniform(0), src_len32(nullptr), src_mapped(nullptr), fused_build(false), pass_bits_override(-1), l2_slice_bytes(48ull << 20), chunk_positions(0), own_list_max(64), st(nullptr), st2(nullptr), build_pending(false), table_counts(nullptr), fa_totals(nullptr), held(0), sm_count(148), have_text(false), n_total(0), shard_begin(0), shard_len(0), own_begin(0), own_end(0),
+        real_gpu() : n_list(0), src_packed(nullptr), src_byte_offsets(nullptr), src_packed_uniform(0), src_len32(nullptr), src_mapped(nullptr), fused_build(false), st(nullptr), st2(nullptr), build_pending(false), table_counts(nullptr), fa_totals(nullptr), held(0), sm_count(148), have_text(false), n_total(0), shard_begin(0), shard_len(0), own_begin(0), own_end(0),
                      nrec(0), fileid(0), have_reads(false), nreads(0), n_usable(0), total_bases(0), W(0), maxlen(0), qual_present(false),
                      F(0), keybits(0), hit_cap(0), host_hits(nullptr), host_hits_cap(0)
         {
@@ -643,7 +638,6 @@ bool build_tables_fused(real_gpu * h, TablePlan * plan)
 {
         uint32_t const hb = h->tab[0].hb, fb = 2 * h->F;
         if ( hb != h->keybits || h->nreads == 0 || plan[0].empty ) return false;
-        if ( getenv("REAL_GPU_NO_FUSED_BUILD") ) return false;
         uint32_t const nlA = table_lists(0, h->prm.seedkmax);
         uint64_t const cap_items = h->nreads * 2 * nlA;
         uint32_t const pbmin = hb > 16 ? hb - 16 : 0, pbmax = std::min<uint32_t>(std::min<uint32_t>(16, hb > 5 ? hb - 5 : 0), fb);
@@ -689,19 +683,15 @@ bool build_tables_fused(real_gpu * h, TablePlan * plan)
         Grouped const GR = partition_entries(h, TP);
         B.item_seed = GR.seed; B.item_val = GR.val; B.sub_start = GR.start;
         B.sub_shift = TP.sub_shift; B.words = TP.words; B.first_sub = TP.first_sub;
-        // one CTA per (sub-bucket, table) by default: three times the CTAs with a third of the shared memory each (measured, r02);
-        // REAL_GPU_BUILD_SPLIT=0: one CTA builds the sub-bucket of all three tables
-        bool split = true;
-        if ( const char * e = getenv("REAL_GPU_BUILD_SPLIT") ) split = atoi(e) != 0;
-        size_t const smem1 = (size_t)(2 * TP.words + (TP.words + 1) / 2) * 4;
-        size_t const smem = split ? smem1 : 3 * smem1;
+        // one CTA per (sub-bucket, table): three times the CTAs with a third of the shared memory each, faster than one CTA
+        // building the sub-bucket of all three tables (measured, r02)
+        size_t const smem = (size_t)(2 * TP.words + (TP.words + 1) / 2) * 4;
         // -l 32: fragments of 8 bases, direct addressing, sub-buckets of 2^16 slots (sub_local_slot)
-        bool const fast = h->F == 8 && hb == 32 && TP.sub_shift == 16 && ! getenv("REAL_GPU_BUILD_GENERAL");
+        bool const fast = h->F == 8 && hb == 32 && TP.sub_shift == 16;
         typedef void (*build_fn)(const Build3Params);
-        build_fn const kb = split ? (fast ? (build_fn)k_build_sub3<true, true> : (build_fn)k_build_sub3<true, false>)
-                                  : (fast ? (build_fn)k_build_sub3<false, true> : (build_fn)k_build_sub3<false, false>);
+        build_fn const kb = fast ? (build_fn)k_build_sub3<true> : (build_fn)k_build_sub3<false>;
         RG_CUDA(cudaFuncSetAttribute(kb, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        kb<<<split ? TP.own_subs * 3 : TP.own_subs, 256, smem, h->st>>>(B);
+        kb<<<TP.own_subs * 3, 256, smem, h->st>>>(B);
         RG_KERNEL_CHECK(); launch_count(h);
         RG_CUDA(cudaMemcpyAsync(&h->table_counts[0], TP.d_total, 16, cudaMemcpyDeviceToHost, h->st));   // items, distinct slots of A, B, C
         h->fused_build = true;
@@ -919,8 +909,6 @@ void fill_scan_params(real_gpu * h, ScanParams & P, int mode)
         P.rec = ptr<uint64_t>(h->rec); P.nrec = h->nrec; P.fileid = h->fileid;
         P.nranks = 1; P.rank = 0; P.bucket_lo[0] = 0; P.bucket_lo[1] = SC_MAX_BUCKETS; P.seg_cap = 0; P.npairs = 0;
         P.own_b_lo = 0; P.own_b_cnt = SC_MAX_BUCKETS;
-        P.hist_pick_max = 0;          // measured: picking is slower than counting whole words at every rank count (r02)
-        if ( const char * e = getenv("REAL_GPU_HIST_PICK") ) P.hist_pick_max = (uint32_t)atoi(e);
         P.nprobed = ptr<unsigned long long>(h->counters) + 4;
         P.mode = mode;
         P.hits = ptr<RawHit>(h->hits_raw);
@@ -973,6 +961,8 @@ void comm_wait(real_gpu * h, uint32_t slot, uint32_t epoch, long long wait_ms)
 // What a scan decides before its chunk loop: the windows it evaluates, the bucket bits, the positions per chunk, its buffers
 // and the shapes of its kernels.  real_gpu_prepare_scan makes the same plan ahead of the match call (prepare = true: the read
 // set is not known yet, the finest bucket split is taken).
+static const uint64_t L2_SLICE_BYTES = 48ull << 20;       // table bytes (presence bits + entries) one bucket may touch
+static const uint32_t OWN_LIST_MAX_BUCKETS = 64;          // bucket shards: own buckets up to which the kept positions are listed first
 struct ScanPlan
 {
         ScanParams P;
@@ -1003,14 +993,11 @@ void plan_scan(real_gpu * h, int mode, bool prepare, ScanPlan & S)
                 if ( P.tab[t].nlists )
                         table_bytes += h->tab[t].bitmap_bytes + h->tab[t].nentries * sizeof(Entry);
         uint32_t bbits = 0;
-        if ( h->pass_bits_override >= 0 )
-                bbits = std::min<uint32_t>((uint32_t)h->pass_bits_override, maxbits);
-        else if ( prepare || h->build_pending )
+        if ( prepare || h->build_pending )
                 bbits = maxbits;
         else
-                while ( bbits < maxbits && (table_bytes >> bbits) > h->l2_slice_bytes ) ++bbits;
+                while ( bbits < maxbits && (table_bytes >> bbits) > L2_SLICE_BYTES ) ++bbits;
         P.bucket_bits = bbits;
-        if ( const char * e = getenv("REAL_GPU_DEBUG") ) P.debug_flags = (uint32_t)atoi(e);
 
         real_gpu::Comm & CM = h->comm;
         bool const sharded = S.sharded = CM.nranks > 1 && CM.window.p;          // records exchanged through peer memory
@@ -1036,12 +1023,12 @@ void plan_scan(real_gpu * h, int mode, bool prepare, ScanPlan & S)
         // Positions partitioned at a time.  One handle with the whole signature space: as many as fit -- the records of
         // C3's 3.1 G positions take 50 GB of the 180 -- because every chunk walks through all the tables again (three chunks
         // of 2^30 positions read the entries three times over: 105 GB of DRAM traffic instead of 10, 2 ms of the C3 scan).
-        // Equal chunks when the text does not fit; REAL_GPU_CHUNK_MPOS overrides.
+        // Equal chunks when the text does not fit.  Sharded tables: the rounds the record areas of the windows were sized for.
         // A bucket shard is sized like a single handle -- all positions of a chunk may fall into its buckets -- plus the 4-byte
         // list of the kept positions: one chunk for C3 on every rank too (r02 up to here: rounds of 2^30 positions).
-        bool const will_list = own_only && P.own_b_cnt <= (uint32_t)h->own_list_max;
-        uint64_t chunk_max = sharded ? CM.round_positions : std::min<uint64_t>(h->chunk_positions, SC_MAX_CHUNK);
-        if ( ! sharded && h->chunk_positions == 0 )
+        bool const will_list = own_only && P.own_b_cnt <= OWN_LIST_MAX_BUCKETS;
+        uint64_t chunk_max = CM.round_positions;
+        if ( ! sharded )
         {
                 uint64_t const span = ((x_end - x_begin + SC_TILE_POS - 1) / SC_TILE_POS) * SC_TILE_POS;
                 uint64_t const pad = (uint64_t)SC_MAX_BUCKETS * SC_UNIT;
@@ -1061,13 +1048,11 @@ void plan_scan(real_gpu * h, int mode, bool prepare, ScanPlan & S)
                 uint64_t const nchunks = (span + fit - 1) / fit;
                 chunk_max = std::max<uint64_t>(SC_TILE_POS, ((span + nchunks - 1) / nchunks + SC_TILE_POS - 1) / SC_TILE_POS * SC_TILE_POS);
         }
-        else if ( h->chunk_positions == 0 )
-                chunk_max = CM.round_positions;
         uint64_t const chunk_cap = S.chunk_cap = std::min<uint64_t>(chunk_max, ((x_end - x_begin + SC_TILE_POS - 1) / SC_TILE_POS) * SC_TILE_POS);
         if ( sharded && prepare ) return;                                        // nothing to form ahead: the caller gives up
         // entries are touched about once per chunk and bucket: several chunks stream them past the probed slot words
         // (evict_first); a single chunk re-uses every entry line about nine times while its bucket is probed (evict_normal)
-        if ( ! getenv("REAL_GPU_DEBUG") && x_end - x_begin <= chunk_cap ) P.debug_flags |= 4;
+        P.entries_evict_normal = x_end - x_begin <= chunk_cap;
         uint32_t * meta = nullptr;
         if ( sharded )
         {
@@ -1127,10 +1112,9 @@ void plan_scan(real_gpu * h, int mode, bool prepare, ScanPlan & S)
         if ( occ_p < 1 ) occ_p = 1;
         if ( occ_s < 1 ) occ_s = 1;
         if ( occ_b < 1 ) occ_b = 1;
-        // more than REAL_PROBE_MINB CTAs per SM make the probe slower (measured: 87 vs 74 ms scan on C3 with four): the grabs
+        // more than SC_PROBE_MINB CTAs per SM make the probe slower (measured: 87 vs 74 ms scan on C3 with four): the grabs
         // of more warps spread over more of the bucket order and the probed slices lose their place in L2
-        if ( occ_b > REAL_PROBE_MINB ) occ_b = REAL_PROBE_MINB;
-        if ( const char * e = getenv("REAL_GPU_PROBE_OCC") ) occ_b = std::max(1, atoi(e));
+        if ( occ_b > SC_PROBE_MINB ) occ_b = SC_PROBE_MINB;
         S.occ_p = occ_p; S.occ_s = occ_s; S.occ_b = occ_b;
         S.wait_ms = 30000;             // a peer that never arrives is reported, not waited for forever
         if ( const char * e = getenv("REAL_GPU_COMM_TIMEOUT_MS") ) S.wait_ms = atoll(e);
@@ -1138,7 +1122,7 @@ void plan_scan(real_gpu * h, int mode, bool prepare, ScanPlan & S)
 
 // the partition kernels of one chunk (P.x_begin .. P.x_end) on stream st: bucket histogram (or the kept-position list of a
 // bucket shard), bucket offsets, staged scatter of the records.  nprobed: where a bucket shard counts the positions it kept.
-void launch_partition(real_gpu * h, ScanPlan const & S, ScanParams const & P, cudaStream_t st, std::function<void()> const & mark)
+void launch_partition(real_gpu * h, ScanPlan const & S, ScanParams const & P, cudaStream_t st)
 {
         real_gpu::Comm & CM = h->comm;
         bool const any = P.x_end > P.x_begin;
@@ -1157,13 +1141,11 @@ void launch_partition(real_gpu * h, ScanPlan const & S, ScanParams const & P, cu
                 k_part_hist<<<pgrid, SC_THREADS, S.psmem, st>>>(P);
                 RG_KERNEL_CHECK(); launch_count(h); h->stats.scan_launches += 1;
         }
-        mark();
         if ( S.sharded )
         {
                 // the owners must have consumed the previous round before their record areas are written again
                 comm_wait(h, 1, CM.epoch - 1, S.wait_ms);
         }
-        mark();
         k_part_offsets<<<1, SC_MAX_BUCKETS, 0, st>>>(P);
         RG_KERNEL_CHECK();
         if ( any )
@@ -1214,7 +1196,7 @@ void prepare_scan(real_gpu * h, uint32_t max_read_len, bool reads_known)
         if ( h->text_pending ) RG_CUDA(cudaStreamWaitEvent(h->st3, h->ev_words, 0));
         RG_CUDA(cudaMemsetAsync(P.nprobed, 0, 8, h->st3));
         RG_CUDA(cudaEventRecord(R.ev0, h->st3));
-        launch_partition(h, S, P, h->st3, [](){});
+        launch_partition(h, S, P, h->st3);
         RG_CUDA(cudaEventRecord(R.done, h->st3));
         R.x_begin = S.x_begin; R.x_end = S.x_end; R.win_begin = P.win_begin; R.win_end = P.win_end; R.chunk_cap = S.chunk_cap;
         R.bucket_bits = P.bucket_bits; R.own_b_lo = P.own_b_lo; R.own_b_cnt = P.own_b_cnt; R.own_list = S.own_list; R.recs = P.recs;
@@ -1233,7 +1215,7 @@ void auto_prepare_scan(real_gpu * h)
         // (a bucket shard keeps a part of the positions of a long text: its filter / list and scatter kernels leave room again --
         // one rank of 2 / 4 / 8 on C3: 51.6 -> 49.0, 28.6 -> 27.4, 15.4 -> 14.9 ms per step)
         bool const light_shard = h->comm.nranks >= 2 && ! h->comm.window.p;
-        if ( h->shard_len > AUTO_PREPARE_MAX_POSITIONS && ! light_shard && ! getenv("REAL_GPU_AUTO_PREPARE") ) return;
+        if ( h->shard_len > AUTO_PREPARE_MAX_POSITIONS && ! light_shard ) return;
         try { prepare_scan(h, h->maxlen, true); }
         catch ( LimitError const & ) { h->prep.valid = false; }
         catch ( CudaError const & ) { cudaGetLastError(); h->prep.valid = false; }          // what is wrong with the set-up is reported by the match call
@@ -1276,14 +1258,9 @@ uint64_t run_scan(real_gpu * h, int mode)
                 else
                         RG_CUDA(cudaMemsetAsync(P.nprobed, 0, 8, h->st));
                 h->stats.n_windows = 0;
-                // REAL_GPU_TRACE=1: per-round phase times on stderr (development)
-                bool const trace = getenv("REAL_GPU_TRACE") != nullptr;
-                std::vector<cudaEvent_t> tev;
-                auto mark = [&]() { if ( trace ) { cudaEvent_t e; cudaEventCreate(&e); cudaEventRecord(e, h->st); tev.push_back(e); } };
                 for ( uint64_t cb = x_begin; cb < x_end; cb += chunk_cap )
                 {
                         if ( nprobe_ev >= 64 ) nprobe_ev = 63;              // (very long texts: the last pairs are re-used)
-                        mark();
                         uint64_t const ce = std::min<uint64_t>(x_end, cb + chunk_cap);
                         P.pos_base = cb;
                         P.x_begin = cb; P.x_end = ce;
@@ -1296,9 +1273,7 @@ uint64_t run_scan(real_gpu * h, int mode)
                                 ++CM.epoch;
                         }
                         if ( ! own_only ) h->stats.n_windows += P.x_end - P.x_begin;
-                        if ( use_prep ) { mark(); mark(); }
-                        else launch_partition(h, S, P, h->st, mark);
-                        mark();
+                        if ( ! use_prep ) launch_partition(h, S, P, h->st);
                         if ( sharded )
                         {
                                 comm_signal(h, 0);
@@ -1306,7 +1281,6 @@ uint64_t run_scan(real_gpu * h, int mode)
                                 k_comm_pairs<<<1, SC_PAIR_THREADS, 0, h->st>>>(P, reinterpret_cast<uint32_t *>(CM.base[CM.rank] + CM.meta_off));
                                 RG_KERNEL_CHECK(); launch_count(h);
                         }
-                        mark();
                         if ( h->evp.size() < 2 * (nprobe_ev + 1) )
                         {
                                 cudaEvent_t a, b;
@@ -1319,7 +1293,6 @@ uint64_t run_scan(real_gpu * h, int mode)
                         RG_KERNEL_CHECK();
                         RG_CUDA(cudaEventRecord(h->evp[2 * nprobe_ev + 1], h->st));
                         ++nprobe_ev;
-                        mark();
                         if ( sharded )
                         {
                                 comm_signal(h, 1);
@@ -1336,17 +1309,6 @@ uint64_t run_scan(real_gpu * h, int mode)
                         R.x_begin = S.x_begin; R.x_end = S.x_end; R.win_begin = P.win_begin; R.win_end = P.win_end; R.chunk_cap = S.chunk_cap;
                         R.bucket_bits = P.bucket_bits; R.own_b_lo = P.own_b_lo; R.own_b_cnt = P.own_b_cnt; R.own_list = S.own_list; R.recs = P.recs;
                         R.valid = true; R.ahead = false;
-                }
-                if ( trace )
-                {
-                        RG_CUDA(cudaStreamSynchronize(h->st));
-                        static const char * names[6] = { "hist", "wait_consumed", "offsets+scatter", "handover", "probe", "" };
-                        for ( size_t i = 0; i + 1 < tev.size(); ++i )
-                        {
-                                if ( i % 6 == 5 ) continue;
-                                fprintf(stderr, "[trace rank %u round %zu] %-16s %8.3f ms\n", CM.rank, i / 6, names[i % 6], elapsed(tev[i], tev[i+1]));
-                        }
-                        for ( cudaEvent_t e : tev ) cudaEventDestroy(e);
                 }
         }
         RG_CUDA(cudaEventRecord(h->ev[6], h->st));
@@ -1388,7 +1350,7 @@ void preload_kernels(int device)
         cudaFuncAttributes a;
 #define RG_PRELOAD(k) RG_CUDA(cudaFuncGetAttributes(&a, k))
         RG_PRELOAD(k_pack_reads); RG_PRELOAD(k_pack_both); RG_PRELOAD(k_seeds_packed); RG_PRELOAD(k_read_seeds); RG_PRELOAD(k_uniform_offsets); RG_PRELOAD(k_flags_to_bad);
-        RG_PRELOAD(k_ent_hist3); RG_PRELOAD(k_ent_offsets); RG_PRELOAD(k_ent_scatter); RG_PRELOAD(k_ent_scatter_own); RG_PRELOAD(k_ent2_hist); RG_PRELOAD(k_ent2_scatter); RG_PRELOAD(k_build_sub); RG_PRELOAD((k_build_sub3<true, true>)); RG_PRELOAD((k_build_sub3<true, false>)); RG_PRELOAD((k_build_sub3<false, true>)); RG_PRELOAD((k_build_sub3<false, false>));
+        RG_PRELOAD(k_ent_hist3); RG_PRELOAD(k_ent_offsets); RG_PRELOAD(k_ent_scatter); RG_PRELOAD(k_ent_scatter_own); RG_PRELOAD(k_ent2_hist); RG_PRELOAD(k_ent2_scatter); RG_PRELOAD(k_build_sub); RG_PRELOAD(k_build_sub3<true>); RG_PRELOAD(k_build_sub3<false>);
         RG_PRELOAD(k_scan_reduce); RG_PRELOAD(k_scan_apply); RG_PRELOAD(k_fill_f32);
         RG_PRELOAD(k_part_hist); RG_PRELOAD(k_part_offsets); RG_PRELOAD(k_part_scatter<false>); RG_PRELOAD(k_part_scatter<true>); RG_PRELOAD(k_own_list); RG_PRELOAD((k_bucket_probe<false, false>)); RG_PRELOAD((k_bucket_probe<true, false>)); RG_PRELOAD((k_bucket_probe<false, true>)); RG_PRELOAD((k_bucket_probe<true, true>));
         RG_PRELOAD(k_comm_signal); RG_PRELOAD(k_comm_wait); RG_PRELOAD(k_comm_pairs);
@@ -1453,11 +1415,7 @@ int real_gpu_create(const real_gpu_params * params, real_gpu ** out)
                 if ( prop.major < 10 ) throw CudaError("device is not sm_100 class; this library only carries sm_100a code");
                 h->sm_count = prop.multiProcessorCount;
                 preload_kernels(params->device);
-                if ( const char * e = getenv("REAL_GPU_PASS_BITS") ) h->pass_bits_override = atoi(e);
-                if ( const char * e = getenv("REAL_GPU_L2_SLICE_MB") ) h->l2_slice_bytes = (uint64_t)atoi(e) << 20;
-                if ( const char * e = getenv("REAL_GPU_OWN_LIST_MAX") ) h->own_list_max = atoi(e);
                 if ( const char * e = getenv("REAL_GPU_AUTO_PREPARE") ) h->auto_prepare = atoi(e) != 0;
-                if ( const char * e = getenv("REAL_GPU_CHUNK_MPOS") ) h->chunk_positions = std::max<uint64_t>(SC_TILE_POS, ((uint64_t)atoi(e) << 20) / SC_TILE_POS * SC_TILE_POS);
                 RG_CUDA(cudaStreamCreateWithFlags(&h->st, cudaStreamNonBlocking));
                 RG_CUDA(cudaStreamCreateWithFlags(&h->st2, cudaStreamNonBlocking));
                 RG_CUDA(cudaMallocHost(&h->table_counts, 6 * sizeof(uint32_t)));

@@ -44,13 +44,8 @@ static const int SC_SMEM_WORDS = SC_TILE_WORDS + 2 * SC_HALO; // 516 words = 412
 static const int SC_MAX_BUCKETS = 256;
 static const int SC_CURSOR_STRIDE = 32;                      // u32 per bucket cursor: one 128-byte line each, so the global atomics spread over the L2 slices
 static const int SC_UNIT = 512;                              // records per grab of the probe kernel (one global atomic per warp and grab)
-#ifndef REAL_SC_RPT
-#define REAL_SC_RPT 2
-#endif
-#ifndef REAL_PROBE_MINB
-#define REAL_PROBE_MINB 3
-#endif
-static const int SC_RPT = REAL_SC_RPT;                       // records per lane and step
+static const int SC_RPT = 2;                                 // records per lane and step
+static const int SC_PROBE_MINB = 3;                          // CTAs per SM of k_bucket_probe (register bound and launch cap, plan_scan)
 static const int SC_QA_CAP = 32 + 96 * SC_RPT;               // per-warp stage A queue (set slot bits): drained from 32 up, a step adds <= 96 per record and lane
 static const int SC_QB_CAP = 64;                             // per-warp stage B queue (seed test passed)
 static const uint32_t SC_POS_NONE = 0xFFFFFFFFu;             // position word of a padding record
@@ -87,7 +82,7 @@ struct ScanParams
         uint32_t fileid;
         // partition of the chunk [x_begin, x_end): x0 = first position of the chunk
         uint32_t bucket_bits;
-        uint32_t debug_flags;         // development only (REAL_GPU_DEBUG): 1 = count set slot bits but do not follow them
+        uint32_t entries_evict_normal;  // 1: the probe loads entries with evict_normal (a single chunk), else evict_first
         uint4 * recs;                 // records grouped by bucket: {window lo, window hi, 16 bases in front of it, position - pos_base}
         uint32_t * bucket_count;      // [SC_MAX_BUCKETS]
         uint32_t * bucket_start;      // [SC_MAX_BUCKETS+1] record index
@@ -114,7 +109,6 @@ struct ScanParams
         // only; it reads every text position of the chunk but forms records only of the positions whose bucket it owns.
         // own_b_cnt = SC_MAX_BUCKETS: no filter.
         uint32_t own_b_lo, own_b_cnt;
-        uint32_t hist_pick_max;       // k_part_hist picks the kept positions out one by one when own_b_cnt <= this
         uint32_t * list;              // bucket shard: positions (relative to pos_base) of the chunk this handle keeps
         unsigned long long * list_count;
         unsigned long long * nprobed; // positions this handle has formed records of (statistics)
@@ -351,11 +345,11 @@ __global__ void __launch_bounds__(SC_THREADS) k_part_hist(ScanParams P)
                         uint32_t const wi = threadIdx.x + k * SC_THREADS;
                         uint64_t const w0 = tw[wi], w1 = tw[wi + 1];
                         uint32_t m = clip_mask(tile_x0 + (uint64_t)wi * 32, P.x_begin, P.x_end);
-                        if ( P.own_b_cnt < SC_MAX_BUCKETS && (P.own_b_cnt <= P.hist_pick_max || ! (m == 0xFFFFFFFFu && bbits == 8)) )
+                        if ( P.own_b_cnt < SC_MAX_BUCKETS && ! (m == 0xFFFFFFFFu && bbits == 8) )
                         {
-                                // bucket shard: only the positions of the own buckets are counted (8-bit buckets).  With many own buckets
-                                // (few ranks) whole words take the path below and count every position -- 32 cheap reductions beat
-                                // picking the kept positions out one by one -- and the counts of foreign buckets are dropped at the end
+                                // bucket shard: only the positions of the own buckets are counted (8-bit buckets).  Whole words take
+                                // the path below and count every position -- 32 cheap reductions beat picking the kept positions out
+                                // one by one at every rank count (measured, r02) -- and the counts of foreign buckets are dropped at the end
                                 uint64_t eq = kept_positions_clipped(w0, w1, P.own_b_lo, P.own_b_cnt, tile_x0 + (uint64_t)wi * 32, P.x_begin, P.x_end);
                                 while ( eq )
                                 {
@@ -400,14 +394,8 @@ __global__ void __launch_bounds__(SC_THREADS) k_part_hist(ScanParams P)
 // of DRAM reads and 5 GB of writes for 3 GB of records, 10 ms per 250 M positions).  Ranks come from a
 // warp-level multisplit (peers_u8 on the bucket id: one ballot per bit): shared-memory atomics that return a value
 // serialise far too much for this.
-#ifndef REAL_PS_PPT
-#define REAL_PS_PPT 8
-#endif
-#ifndef REAL_PS_THREADS
-#define REAL_PS_THREADS 256
-#endif
-static const int PS_THREADS = REAL_PS_THREADS;                // threads per CTA (256 or 512); the first 256 also act for one bucket each
-static const int PS_PPT = REAL_PS_PPT;                        // positions per thread (4, 8, 16 or 32)
+static const int PS_THREADS = 256;                            // threads per CTA (256 or 512); the first 256 also act for one bucket each
+static const int PS_PPT = 8;                                  // positions per thread (4, 8, 16 or 32)
 static const int PS_TPW = 32 / PS_PPT;                            // threads per text word
 static const int PS_TILE_POS = PS_THREADS * PS_PPT;           // 2048 (4096 with 512 threads)
 static const int PS_TILE_WORDS = PS_TILE_POS / 32;            // 128
@@ -1060,9 +1048,10 @@ __device__ __forceinline__ uint32_t drain_a_warp(ScanParams const & P, ProbeSmem
         ItemB * qb = S.qb[wid];
         uint32_t * qbn = &S.qbn[wid];
         uint32_t lstats[3] = {0, 0, 0};
-        // entries are touched about once per bucket pass: by default they go through L2 with evict_first priority so
-        // that they do not push the presence words (probed several times per line) out of the protected set
-        uint64_t const pol_e = (P.debug_flags & 2) ? policy_evict_last() : ((P.debug_flags & 4) ? policy_evict_normal() : policy_evict_first());
+        // entries are touched about once per bucket pass: when several chunks stream them past, they go through L2 with
+        // evict_first priority so that they do not push the presence words (probed several times per line) out of the
+        // protected set (plan_scan)
+        uint64_t const pol_e = P.entries_evict_normal ? policy_evict_normal() : policy_evict_first();
         while ( n >= 32 || (flush && n) )
         {
                 uint32_t const take = n >= 32 ? 32u : n;
@@ -1097,7 +1086,7 @@ __device__ __forceinline__ const uint4 * grab_records(ScanParams const & P, uint
 
 // WIDE: seeds longer than the indexed 32 bases (the whole-seed test costs registers the common case must not pay for)
 template<bool WIDE, bool PACKED>
-__global__ void __launch_bounds__(SC_THREADS, REAL_PROBE_MINB) k_bucket_probe(const __grid_constant__ ScanParams P)
+__global__ void __launch_bounds__(SC_THREADS, SC_PROBE_MINB) k_bucket_probe(const __grid_constant__ ScanParams P)
 {
         extern __shared__ __align__(128) unsigned char sc_smem[];
         ProbeSmem & S = *reinterpret_cast<ProbeSmem *>(sc_smem);
@@ -1186,7 +1175,6 @@ __global__ void __launch_bounds__(SC_THREADS, REAL_PROBE_MINB) k_bucket_probe(co
                                         cand |= ((cur[k].w != SC_POS_NONE) ? ((sw[k][t].bits >> ((bits5[k] >> (5 * t)) & 31)) & 1u) : 0u) << (k * 3 + t);
                         if ( __any_sync(0xffffffffu, cand != 0) )
                         {
-                                uint32_t const n0 = qn;
                                 #pragma unroll
                                 for ( int k = 0; k < SC_RPT; ++k )
                                         #pragma unroll
@@ -1205,12 +1193,7 @@ __global__ void __launch_bounds__(SC_THREADS, REAL_PROBE_MINB) k_bucket_probe(co
                                                 qn += __popc(bal);
                                         }
                                 __syncwarp();
-                                if ( P.debug_flags & 1 )
-                                {
-                                        if ( lane == 0 ) S.stat[0][threadIdx.x] += qn - n0;
-                                        qn = 0;
-                                }
-                                else if ( qn >= 32 )
+                                if ( qn >= 32 )
                                         qn = drain_a_warp<WIDE, PACKED>(P, S, qn, false);
                         }
                 }
