@@ -5,6 +5,7 @@ import numpy as np
 import pytest
 
 from real_b200 import lib as rlib, matcher, synth
+from util import line as _line, read_bases as _bases
 
 pytestmark = pytest.mark.gpu
 
@@ -25,18 +26,6 @@ def test_score_formatter_equals_printf_g():
     want = [("%g" % float(x)).encode() for x in v]
     bad = [(float(x), g, w) for x, g, w in zip(v, got, want) if g != w]
     assert not bad, bad[:10]
-
-
-def _line(idb, bases, score, L, inverted, name, pos1, k):
-    s = idb + b"\t" + bases + b"\t" + (("%g" % float(score)).encode() if score is not None else b"") + b"\t1\ta\t" + str(L).encode()
-    return s + (b"\t-\t" if inverted else b"\t+\t") + name + b"\t" + str(pos1).encode() + b"\t\t" + str(k).encode() + b"\n"
-
-
-def _bases(reads, r, inverted):
-    m = reads.read(r)
-    if inverted:
-        m = synth.revcomp_mapped(m)
-    return bytes(b"ACGTN"[int(x)] for x in m)
 
 
 @pytest.mark.parametrize("scores", [False, True])

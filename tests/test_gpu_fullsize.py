@@ -19,18 +19,11 @@ import pytest
 
 from real_b200 import lib as rlib
 from real_b200 import matcher
+from util import need_big_gpu as _need_big_gpu
 
 pytestmark = pytest.mark.gpu
 
 SEED = 0x5EA1
-
-
-def _need_big_gpu(gb):
-    import torch
-    if not torch.cuda.is_available():
-        pytest.skip("no GPU")
-    if torch.cuda.get_device_properties(0).total_memory < gb * (1 << 30):
-        pytest.skip("needs a GPU with %d GB" % gb)
 
 
 def _record_starts(n, nrec):

@@ -74,6 +74,33 @@ def unify_order_ok(h) -> bool:
     return True
 
 
+def need_big_gpu(gb, free_gb=0):
+    """Skips the calling test unless device 0 has `gb` GB in all and, when given, `free_gb` GB free right now."""
+    import pytest
+    import torch
+    if not torch.cuda.is_available():
+        pytest.skip("no GPU")
+    if torch.cuda.get_device_properties(0).total_memory < gb * (1 << 30):
+        pytest.skip("needs a GPU with %d GB" % gb)
+    if free_gb and torch.cuda.mem_get_info(0)[0] < free_gb * (1 << 30):
+        pytest.skip("needs %d GB of free device memory" % free_gb)
+
+
+def line(idb, bases, score, L, inverted, name, pos1, k):
+    """One output line of a hit as the reference prints it (read id, bases on the hit's strand, score, record name,
+    1-based position in the record, errors)."""
+    s = idb + b"\t" + bases + b"\t" + (("%g" % float(score)).encode() if score is not None else b"") + b"\t1\ta\t" + str(L).encode()
+    return s + (b"\t-\t" if inverted else b"\t+\t") + name + b"\t" + str(pos1).encode() + b"\t\t" + str(k).encode() + b"\n"
+
+
+def read_bases(reads, r, inverted):
+    """The bases of read r as ACGTN text, reverse complemented for a '-' hit."""
+    m = reads.read(r)
+    if inverted:
+        m = synth.revcomp_mapped(m)
+    return bytes(b"ACGTN"[int(x)] for x in m)
+
+
 def text_quirk_cases():
     """[(name, fasta bytes, symbols, starts incl. terminal, [names])] of tests/golden/text_quirks.npz (the reference's own getText)."""
     z = np.load(os.path.join(GOLDEN, "text_quirks.npz"))
