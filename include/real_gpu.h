@@ -345,7 +345,8 @@ int real_gpu_fold_unique_group(real_gpu * const * handles, uint32_t n);
  *   real_gpu_comm_connect        all_handles = the nranks handles in rank order (one process per GPU)
  *   real_gpu_comm_connect_local  the same for ranks that live in one process (peers = the nranks handles)
  * All ranks must use the same round_positions and make the same sequence of match calls.  Order dependent folds
- * (matchUnique with scores, real_gpu_match_gaps) are not available in this mode. */
+ * (matchUnique with scores, real_gpu_match_gaps) are not available in this mode.  Seeds of fewer than 16 bases are
+ * refused (REAL_GPU_E_ARG, the handle is left as it was): they have fewer than 256 scan buckets to split. */
 #define REAL_GPU_COMM_HANDLE_BYTES 64
 int real_gpu_comm_init(real_gpu * h, uint32_t rank, uint32_t nranks, uint64_t round_positions, void * handle_out);
 int real_gpu_comm_connect(real_gpu * h, const void * all_handles);
@@ -358,7 +359,8 @@ int real_gpu_comm_connect_local(real_gpu * h, real_gpu * const * peers);
  * of the index build, of the record traffic and of the probes.  Every hit is found by exactly one rank; matchAll
  * results are the union of the ranks' results, matchUnique states are merged with the real_gpu_unique_export_*
  * exchange above -- the only cross-GPU traffic of the path.  Call before real_gpu_set_reads.  Order dependent folds
- * (matchUnique with scores, real_gpu_match_gaps) are not available in this mode. */
+ * (matchUnique with scores, real_gpu_match_gaps) are not available in this mode.  Seeds of fewer than 16 bases are
+ * refused (REAL_GPU_E_ARG, the handle is left as it was): they have fewer than 256 scan buckets to split. */
 int real_gpu_set_bucket_shard(real_gpu * h, uint32_t rank, uint32_t nranks);
 
 /* Gapped extension pass (UniqueMatcher::matchGaps) for reads still NoMatch/Gapped; updates the

@@ -445,7 +445,9 @@ static uint32_t * enumerate_windows(const oracle_text * T, uint32_t seedl, uint6
  * per read context (RestWordBuffer.hpp:33-78, RestMatch.hpp:84-111)
  * ---------------------------------------------------------------------------------------- */
 
-#define ORACLE_MAX_REST_WORDS 64
+/* reads of up to 65535 bases (the product's limit): the rest of the read is at most 65535 - 4 bases, 2048 words.
+ * Two such buffers make read_ctx 32 KB, well inside a thread's stack. */
+#define ORACLE_MAX_REST_WORDS 2048
 
 typedef struct
 {

@@ -2344,6 +2344,8 @@ int real_gpu_comm_init(real_gpu * h, uint32_t rank, uint32_t nranks, uint64_t ro
 {
         RG_API_BEGIN(h)
         if ( nranks < 1 || nranks > (uint32_t)SC_MAX_RANKS || rank >= nranks ) return fail(h, REAL_GPU_E_ARG, "comm_init: rank/nranks out of range (at most 8 ranks)");
+        // the ranks split the 256 scan buckets (the first 4 bases of a seed window): a seed of 4..12 bases has fewer
+        if ( nranks > 1 && h->prm.seedl < 16 ) return fail(h, REAL_GPU_E_ARG, "comm_init: sharded tables need seeds of at least 16 bases");
         real_gpu::Comm & CM = h->comm;
         if ( CM.window.p ) return fail(h, REAL_GPU_E_STATE, "comm_init: already initialised");
         drop_prepared(h);
@@ -2384,6 +2386,8 @@ int real_gpu_set_bucket_shard(real_gpu * h, uint32_t rank, uint32_t nranks)
 {
         RG_API_BEGIN(h)
         if ( nranks < 1 || nranks > (uint32_t)SC_MAX_RANKS || rank >= nranks ) return fail(h, REAL_GPU_E_ARG, "set_bucket_shard: rank/nranks out of range (at most 8 ranks)");
+        // the ranks split the 256 scan buckets (the first 4 bases of a seed window): a seed of 4..12 bases has fewer
+        if ( nranks > 1 && h->prm.seedl < 16 ) return fail(h, REAL_GPU_E_ARG, "set_bucket_shard: bucket shards need seeds of at least 16 bases");
         real_gpu::Comm & CM = h->comm;
         if ( CM.window.p ) return fail(h, REAL_GPU_E_STATE, "set_bucket_shard: the handle is already a rank of a peer-memory group (real_gpu_comm_init)");
         drop_prepared(h);

@@ -74,6 +74,16 @@ def unify_order_ok(h) -> bool:
     return True
 
 
+def fresh(seed, n=1_500_000, nreads=40_000, L=100, nrec=7, npm=1500, sub=0.012, fastq=True):
+    """A random text with a 20 kbp repeat (reads with several hits) and genpat reads drawn from it."""
+    text = synth.make_text(seed, n, nrecords=nrec, n_per_million=npm)
+    sym = text.symbols.copy()
+    sym[n // 2:n // 2 + 20000] = sym[1000:21000]          # a repeat => multi-hit reads
+    text = synth.Text(sym, text.records)
+    reads = synth.make_reads(text, seed + 1, nreads, L, sub, fastq=fastq)
+    return text, reads
+
+
 def need_big_gpu(gb, free_gb=0):
     """Skips the calling test unless device 0 has `gb` GB in all and, when given, `free_gb` GB free right now."""
     import pytest
