@@ -298,6 +298,11 @@ int real_gpu_reset_unique(real_gpu * h);
  * as its memory planner would choose them (matchUniqueImplementation.cpp:1208-1244); 0 = one block per file.
  * Also used by real_gpu_match_gaps.  In this mode the handle must hold the whole file (one shard). */
 int real_gpu_set_block_windows(real_gpu * h, uint64_t n_list);
+/* Test hook: the reference text blocks the order dependent folds would use on the current text with n_list windows per
+ * block.  *nblocks receives their number (1 when n_list is 0 or the text has at most n_list seed windows) and
+ * bounds[0 .. min(nblocks, cap)) the position of the first seed window of each block (bounds[0] = 0).  The handle's own
+ * n_list (real_gpu_set_block_windows) is left as it was.  Needs the whole file in one shard. */
+int real_gpu_get_block_bounds(real_gpu * h, uint64_t n_list, uint64_t * bounds, uint64_t cap, uint64_t * nblocks);
 
 /* Cross-shard exchange for matchUnique without scores (SURVEY.md 8e): the per-read state is
  * exported as an order-preserving u64 key so that a MIN all-reduce followed by a SUM all-reduce of

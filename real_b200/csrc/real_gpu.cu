@@ -2226,6 +2226,29 @@ int real_gpu_set_block_windows(real_gpu * h, uint64_t n_list)
         return REAL_GPU_OK;
 }
 
+int real_gpu_get_block_bounds(real_gpu * h, uint64_t n_list, uint64_t * bounds, uint64_t cap, uint64_t * nblocks)
+{
+        RG_API_BEGIN(h)
+        if ( ! nblocks || (cap && ! bounds) ) return fail(h, REAL_GPU_E_ARG, "get_block_bounds: null pointer");
+        if ( ! h->have_text ) return fail(h, REAL_GPU_E_STATE, "no text set");
+        if ( h->shard_begin != 0 || h->shard_len != h->n_total )
+                return fail(h, REAL_GPU_E_ARG, "get_block_bounds needs the whole file in one shard");
+        uint64_t const saved = h->n_list;
+        h->n_list = n_list;
+        uint32_t nb = 1;
+        try { nb = block_bounds(h); } catch ( ... ) { h->n_list = saved; throw; }
+        h->n_list = saved;
+        *nblocks = nb;
+        if ( cap ) bounds[0] = 0;
+        if ( nb > 1 && cap > 1 )
+        {
+                RG_CUDA(cudaMemcpyAsync(bounds, ptr<uint64_t>(h->bounds), std::min<uint64_t>(nb, cap) * 8, cudaMemcpyDeviceToHost, h->st));
+                RG_CUDA(cudaStreamSynchronize(h->st));
+        }
+        return REAL_GPU_OK;
+        RG_API_END(h)
+}
+
 int real_gpu_unique_export_keys(real_gpu * h, uint64_t * d_keys)
 {
         RG_API_BEGIN(h)

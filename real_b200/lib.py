@@ -110,6 +110,7 @@ def load(build_if_missing: bool = True):
     L.real_gpu_reset_unique.argtypes = [vp]
     L.real_gpu_unique_checksum.argtypes = [vp, u64, u64, C.POINTER(u64)]
     L.real_gpu_set_block_windows.argtypes = [vp, u64]
+    L.real_gpu_get_block_bounds.argtypes = [vp, u64, vp, u64, C.POINTER(u64)]
     L.real_gpu_unique_export_keys.argtypes = [vp, vp]
     L.real_gpu_unique_export_ties.argtypes = [vp, vp, vp]
     L.real_gpu_unique_import.argtypes = [vp, vp, vp]
@@ -393,6 +394,14 @@ class Handle:
 
     def set_block_windows(self, n_list: int):
         self._check(self.L.real_gpu_set_block_windows(self.h, n_list))
+
+    def get_block_bounds(self, n_list: int, cap: int = 1 << 16) -> np.ndarray:
+        """Position of the first seed window of every reference text block of the current text at n_list windows per block."""
+        b = np.zeros(cap, dtype=np.uint64)
+        nb = C.c_uint64()
+        self._check(self.L.real_gpu_get_block_bounds(self.h, n_list, b.ctypes.data, cap, C.byref(nb)))
+        assert nb.value <= cap, (nb.value, cap)
+        return b[:nb.value]
 
     def unique_export_keys(self, d_keys: int):
         self._check(self.L.real_gpu_unique_export_keys(self.h, d_keys))

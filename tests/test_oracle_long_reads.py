@@ -6,7 +6,7 @@ import pytest
 
 from oracle import oracle_py as O
 from real_b200 import synth
-from util import canon_hits
+from util import brute_match_all, canon_hits
 
 
 def long_read_case(seed, seedl):
@@ -51,45 +51,6 @@ def long_read_case(seed, seedl):
     plant(4099, 68_000, 0, 0, valid=False)                # window across the record boundary at 70000
     plant(4099, 98_000, 1, 0, valid=False)                # window over the N run
     return text, synth.reads_from_list(seqs, quals), plan
-
-
-def brute_match_all(text, reads, seedl, s, e, ll):
-    sym = text.symbols
-    n = text.n
-    starts = text.record_starts.astype(np.int64)
-    cum_n = np.concatenate([[0], np.cumsum(sym > 3)])
-    rows = []
-    for r in range(reads.nreads):
-        rd, q = reads.read(r), reads.qual(r)
-        L = len(rd)
-        if L < seedl or L > n or (rd > 3).any():
-            continue
-        nwin = n - L + 1
-        for inv in (0, 1):
-            fwd = synth.revcomp_mapped(rd) if inv else rd
-            qq = q[::-1] if inv else q
-            sa = L - seedl if inv else 0
-            seedk = np.zeros(nwin, np.int32)
-            for j in range(sa, sa + seedl):               # the seed's mismatches at every window
-                seedk += sym[j:j + nwin] != fwd[j]
-            for p in np.nonzero(seedk <= s)[0]:
-                p = int(p)
-                if cum_n[p + L] != cum_n[p]:
-                    continue
-                rec = int(np.searchsorted(starts, p, "right")) - 1
-                if p + L > starts[rec + 1]:
-                    continue
-                win = sym[p:p + L]
-                k = int((win != fwd).sum())
-                if k > e:
-                    continue
-                idx = ((win.astype(np.int64) << 8) | (fwd.astype(np.int64) << 6) | qq) & 1023
-                raw = 1.0
-                for v in ll[idx].tolist():               # in read order, as the reference adds them
-                    raw += v
-                rows.append((r, k, p, 0, rec, inv, int(np.float32(raw).view(np.uint32))))
-    a = np.asarray(rows, dtype=np.int64).reshape(-1, 7)
-    return a[np.lexsort(a.T[::-1])]
 
 
 @pytest.mark.parametrize("seedl,s,e", [(32, 2, 12), (12, 2, 15), (64, 1, 9)])
