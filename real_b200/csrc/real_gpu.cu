@@ -1084,11 +1084,12 @@ void plan_scan(real_gpu * h, int mode, bool prepare, ScanPlan & S)
         P.unit_counter = meta + 256 + 520;
         P.bucket_cursor = meta + 1088;
 
-        S.psmem = sizeof(HistSmem); S.ssmem = sizeof(ScatterSmem); S.bsmem = sizeof(ProbeSmem);
+        S.psmem = sizeof(HistSmem); S.bsmem = sizeof(ProbeSmem);
         // Bucket shard: with few own buckets (four ranks or more) one light pass lists the kept positions and counts them per
         // bucket, and the staged scatter runs on the list; with many (two ranks: half of all positions are kept) listing
         // costs more than it saves, and the dense kernels run with a filter on the bucket (measured, profiles/r02_*)
         bool const own_list = S.own_list = will_list;
+        S.ssmem = own_list ? sizeof(ListScatterSmem) : sizeof(ScatterSmem);
         if ( own_list )
         {
                 // the positions of a chunk this rank keeps, 4 bytes each (all of them if the text falls into its buckets only)
@@ -1097,8 +1098,7 @@ void plan_scan(real_gpu * h, int mode, bool prepare, ScanPlan & S)
                 P.list_count = reinterpret_cast<unsigned long long *>(meta + 780);
         }
         RG_CUDA(cudaFuncSetAttribute(k_part_hist, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S.psmem));
-        RG_CUDA(cudaFuncSetAttribute(k_part_scatter<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S.ssmem));
-        RG_CUDA(cudaFuncSetAttribute(k_part_scatter<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S.ssmem));
+        RG_CUDA(cudaFuncSetAttribute(own_list ? (const void *)k_part_scatter_list : (const void *)k_part_scatter, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S.ssmem));
         bool const wide = h->prm.seedl > 32;
         typedef ScanPlan::probe_fn probe_fn;
         bool const packed_src = h->src_packed != nullptr;
@@ -1107,7 +1107,8 @@ void plan_scan(real_gpu * h, int mode, bool prepare, ScanPlan & S)
         RG_CUDA(cudaFuncSetAttribute(S.probe, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S.bsmem));
         int occ_p = 0, occ_b = 0, occ_s = 0;
         RG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_p, k_part_hist, SC_THREADS, S.psmem));
-        RG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_s, own_list ? k_part_scatter<true> : k_part_scatter<false>, PS_THREADS, S.ssmem));
+        if ( own_list ) RG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_s, k_part_scatter_list, PS_THREADS, S.ssmem));
+        else RG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_s, k_part_scatter, PD_THREADS, S.ssmem));
         RG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_b, S.probe, SC_THREADS, S.bsmem));
         if ( occ_p < 1 ) occ_p = 1;
         if ( occ_s < 1 ) occ_s = 1;
@@ -1150,12 +1151,12 @@ void launch_partition(real_gpu * h, ScanPlan const & S, ScanParams const & P, cu
         RG_KERNEL_CHECK();
         if ( any )
         {
-                uint64_t const sft = P.x_begin / PS_TILE_POS, set = (P.x_end + PS_TILE_POS - 1) / PS_TILE_POS;
+                uint64_t const sft = P.x_begin / PD_TILE_POS, set = (P.x_end + PD_TILE_POS - 1) / PD_TILE_POS;
                 unsigned const sgrid = (unsigned)std::min<uint64_t>(set - sft, (uint64_t)h->sm_count * S.occ_s);
                 if ( S.own_list )
-                        k_part_scatter<true><<<(unsigned)(h->sm_count * S.occ_s), PS_THREADS, S.ssmem, st>>>(P);
+                        k_part_scatter_list<<<(unsigned)(h->sm_count * S.occ_s), PS_THREADS, S.ssmem, st>>>(P);
                 else
-                        k_part_scatter<false><<<sgrid, PS_THREADS, S.ssmem, st>>>(P);
+                        k_part_scatter<<<sgrid, PD_THREADS, S.ssmem, st>>>(P);
                 RG_KERNEL_CHECK(); launch_count(h); h->stats.scan_launches += 1;
         }
         launch_count(h);               // k_part_offsets
@@ -1352,7 +1353,7 @@ void preload_kernels(int device)
         RG_PRELOAD(k_pack_reads); RG_PRELOAD(k_pack_both); RG_PRELOAD(k_seeds_packed); RG_PRELOAD(k_read_seeds); RG_PRELOAD(k_uniform_offsets); RG_PRELOAD(k_flags_to_bad);
         RG_PRELOAD(k_ent_hist3); RG_PRELOAD(k_ent_offsets); RG_PRELOAD(k_ent_scatter); RG_PRELOAD(k_ent_scatter_own); RG_PRELOAD(k_ent2_hist); RG_PRELOAD(k_ent2_scatter); RG_PRELOAD(k_build_sub); RG_PRELOAD(k_build_sub3<true>); RG_PRELOAD(k_build_sub3<false>);
         RG_PRELOAD(k_scan_reduce); RG_PRELOAD(k_scan_apply); RG_PRELOAD(k_fill_f32);
-        RG_PRELOAD(k_part_hist); RG_PRELOAD(k_part_offsets); RG_PRELOAD(k_part_scatter<false>); RG_PRELOAD(k_part_scatter<true>); RG_PRELOAD(k_own_list); RG_PRELOAD((k_bucket_probe<false, false>)); RG_PRELOAD((k_bucket_probe<true, false>)); RG_PRELOAD((k_bucket_probe<false, true>)); RG_PRELOAD((k_bucket_probe<true, true>));
+        RG_PRELOAD(k_part_hist); RG_PRELOAD(k_part_offsets); RG_PRELOAD(k_part_scatter); RG_PRELOAD(k_part_scatter_list); RG_PRELOAD(k_own_list); RG_PRELOAD((k_bucket_probe<false, false>)); RG_PRELOAD((k_bucket_probe<true, false>)); RG_PRELOAD((k_bucket_probe<false, true>)); RG_PRELOAD((k_bucket_probe<true, true>));
         RG_PRELOAD(k_comm_signal); RG_PRELOAD(k_comm_wait); RG_PRELOAD(k_comm_pairs);
         RG_PRELOAD(k_score_hits); RG_PRELOAD(k_hit_count); RG_PRELOAD(k_hit_scatter); RG_PRELOAD(k_hit_order<real_gpu_hit>);
         RG_PRELOAD(k_unique_export); RG_PRELOAD(k_unique_ties); RG_PRELOAD(k_unique_import); RG_PRELOAD(k_unique_replay); RG_PRELOAD(k_fold_push); RG_PRELOAD(k_fold_merge); RG_PRELOAD(k_unique_checksum); RG_PRELOAD(k_mark_large); RG_PRELOAD(k_sort_large<0>); RG_PRELOAD(k_sort_large<1>); RG_PRELOAD(k_sort_large<2>);

@@ -20,7 +20,7 @@
 //   k_part_scatter  TMA-staged text tiles -> 16-byte records {window word, the 16 bases in front of it,
 //                   position} grouped by bucket (staged in shared memory, written run by run)
 //   k_own_list      bucket shards (multi-GPU): the positions whose bucket this rank owns, as a dense list + their
-//                   bucket histogram in one pass; k_part_scatter<true> then forms the records of the list
+//                   bucket histogram in one pass; k_part_scatter_list then forms the records of the list
 //   k_bucket_probe  warps pull 512-record grabs in bucket order and walk them 64 records at a time:
 //                   6 independent 4-byte probes per lane; set slot bits are compacted
 //                   into the warp's shared-memory queue (stage A: rank -> entry chain -> seed test ->
@@ -387,42 +387,240 @@ __global__ void __launch_bounds__(SC_THREADS) k_part_hist(ScanParams P)
 }
 
 // ---- partition, scatter pass ---------------------------------------------------------------------
-// Tiles of 4096 positions (half a text word per thread).  Records are first laid out bucket by bucket in
-// shared memory and then copied out run by run, so every global store instruction writes whole
-// consecutive records of one bucket: scattering records straight from the threads that produce them
-// leaves ~200 KB of half-written lines open per CTA, more than L2 holds for a full grid (measured: 2 GB
-// of DRAM reads and 5 GB of writes for 3 GB of records, 10 ms per 250 M positions).  Ranks come from a
-// warp-level multisplit (peers_u8 on the bucket id: one ballot per bit): shared-memory atomics that return a value
-// serialise far too much for this.
-static const int PS_THREADS = 256;                            // threads per CTA (256 or 512); the first 256 also act for one bucket each
-static const int PS_PPT = 8;                                  // positions per thread (4, 8, 16 or 32)
-static const int PS_TPW = 32 / PS_PPT;                            // threads per text word
-static const int PS_TILE_POS = PS_THREADS * PS_PPT;           // 2048 (4096 with 512 threads)
-static const int PS_TILE_WORDS = PS_TILE_POS / 32;            // 128
-static const int PS_SMEM_WORDS = PS_TILE_WORDS + 2 * SC_HALO; // 132 words = 1056 bytes
+// Records are first laid out bucket by bucket in shared memory and then copied out run by run, so every global store
+// instruction writes whole consecutive records of one bucket: scattering records straight from the threads that produce
+// them leaves ~200 KB of half-written lines open per CTA, more than L2 holds for a full grid (measured: 2 GB of DRAM reads
+// and 5 GB of writes for 3 GB of records, 10 ms per 250 M positions).  Ranks come from a warp-level multisplit (peers_u8
+// on the bucket id: one ballot per bit): shared-memory atomics that return a value serialise far too much for this.
+//
+// Dense form (every position of the chunk, or those of the own buckets of a two-rank bucket shard): tiles of 8192
+// positions, one text word per thread.  What is staged is the 2-byte offset of a position in its tile, not its 16-byte
+// record: the copy-out rebuilds the record from the text words of the tile, which are in shared memory anyway.  Staging
+// costs 4 bytes of shared-memory traffic per record instead of 32, and the small staging array lets a tile be four times
+// as large as with staged records, so the per-tile bucket work and barriers are paid four times less often per position
+// and a bucket's run in a tile is ~32 records (whole lines) instead of ~8 (measured, DESIGN 4.3).
+static const int PD_THREADS = 256;                            // threads per CTA; thread b also acts for bucket b
+static const int PD_MINB = 4;                                 // CTAs per SM (64 registers)
+static const int PD_TILE_WORDS = PD_THREADS;                  // one text word per thread
+static const int PD_TILE_POS = PD_TILE_WORDS * 32;            // 8192
+static const int PD_SMEM_WORDS = PD_TILE_WORDS + 2 * SC_HALO; // 260 words = 2080 bytes
+static_assert(PD_THREADS == SC_MAX_BUCKETS, "the bucket work gives every thread one bucket");
+static_assert(SC_TILE_POS % PD_TILE_POS == 0, "a tile must not reach past the last tile of k_part_hist (the text padding)");
+static_assert(PD_TILE_POS <= 65536, "tile offsets are staged in 16 bits");
 
 struct ScatterSmem
 {
-        uint4 stage[PS_TILE_POS];                          // record, position field relative to the tile
-        uint64_t tile[2][PS_SMEM_WORDS];
+        uint64_t tile[2][PD_SMEM_WORDS];                   // bulk-copy destinations first: 16-byte aligned
         uint64_t bar[2];
-        uint32_t wcnt[PS_THREADS / 32][SC_MAX_BUCKETS];    // per-warp counts, then running slots
-        uint32_t loc[SC_MAX_BUCKETS + 1];                  // first staging slot of a bucket
-        uint32_t wsum[SC_MAX_BUCKETS / 32];                // bucket totals per warp of bucket threads (exclusive scan)
         uint4 * dst[SC_MAX_BUCKETS];                       // per tile: record area of the bucket's owner + first record of the tile's run - first staging slot
         uint4 * area[SC_MAX_BUCKETS];                      // record area of the bucket's owner
+        uint32_t wcnt[PD_THREADS / 32][SC_MAX_BUCKETS];    // per-warp counts, then running slots
+        uint32_t loc[SC_MAX_BUCKETS + 1];                  // first staging slot of a bucket
+        uint32_t wsum[SC_MAX_BUCKETS / 32];                // bucket totals per warp of bucket threads (exclusive scan)
+        uint16_t stage[PD_TILE_POS];                       // offset of the position in the tile, bucket-major
 };
 
-// LIST: the positions come from the kept-position list of a bucket shard (k_own_list) instead of the text tiles
-template<bool LIST>
-__global__ void __launch_bounds__(PS_THREADS, 1024 / PS_THREADS) k_part_scatter(ScanParams P)
+// the bucket of base j of the text word w0 (w1 = the word behind it): the top bits of the 16 bases from j on
+__device__ __forceinline__ uint32_t bucket_at(uint64_t w0, uint64_t w1, uint32_t j, uint32_t bsh, uint32_t bmask)
+{
+        uint32_t const top = j < 16 ? __funnelshift_l((uint32_t)w0, (uint32_t)(w0 >> 32), 2 * j)
+                                    : __funnelshift_l((uint32_t)(w1 >> 32), (uint32_t)w0, 2 * j - 32);
+        return (top >> bsh) & bmask;
+}
+
+__global__ void __launch_bounds__(PD_THREADS, PD_MINB) k_part_scatter(ScanParams P)
 {
         extern __shared__ __align__(128) unsigned char sc_smem[];
         ScatterSmem & S = *reinterpret_cast<ScatterSmem *>(sc_smem);
 
-        uint64_t const nlist = LIST ? *P.list_count : 0;
-        uint64_t const first_tile = LIST ? 0 : P.x_begin / PS_TILE_POS;
-        uint64_t const end_tile = LIST ? (nlist + PS_TILE_POS - 1) / PS_TILE_POS : (P.x_end + PS_TILE_POS - 1) / PS_TILE_POS;
+        uint64_t const first_tile = P.x_begin / PD_TILE_POS;
+        uint64_t const end_tile = (P.x_end + PD_TILE_POS - 1) / PD_TILE_POS;
+        uint32_t const bbits = P.bucket_bits;
+        uint32_t const bsh = 32 - (bbits ? bbits : 1);
+        uint32_t const bmask = bbits ? 0xFFFFFFFFu : 0u;
+        uint32_t const fsh = 64 - 2 * P.seedl;
+        bool const filter = P.own_b_cnt < SC_MAX_BUCKETS;          // bucket shard: only the positions of the own buckets
+        int const lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+        uint32_t const lt = (1u << lane) - 1;
+
+        if ( threadIdx.x == 0 )
+        {
+                mbar_init(&S.bar[0], 1);
+                mbar_init(&S.bar[1], 1);
+                asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        }
+        #pragma unroll
+        for ( int w = 0; w < PD_THREADS / 32; ++w ) S.wcnt[w][threadIdx.x] = 0;
+        S.area[threadIdx.x] = P.peer_recs[bucket_owner(P, threadIdx.x)];
+        __syncthreads();
+
+        uint64_t tile_id = first_tile + blockIdx.x;
+        if ( threadIdx.x == 0 && tile_id < end_tile )
+        {
+                mbar_expect_tx(&S.bar[0], PD_SMEM_WORDS * 8);
+                bulk_load(&S.tile[0][0], P.text + (int64_t)tile_id * PD_TILE_WORDS - SC_HALO, PD_SMEM_WORDS * 8, &S.bar[0]);
+        }
+
+        for ( uint32_t it = 0; tile_id < end_tile; tile_id += gridDim.x, ++it )
+        {
+                uint32_t const buf = it & 1;
+                uint64_t const next_tile = tile_id + gridDim.x;
+                if ( threadIdx.x == 0 && next_tile < end_tile )
+                {
+                        mbar_expect_tx(&S.bar[buf ^ 1], PD_SMEM_WORDS * 8);
+                        bulk_load(&S.tile[buf ^ 1][0], P.text + (int64_t)next_tile * PD_TILE_WORDS - SC_HALO, PD_SMEM_WORDS * 8, &S.bar[buf ^ 1]);
+                }
+                mbar_wait(&S.bar[buf], (it >> 1) & 1);
+                const uint64_t * tw = &S.tile[buf][SC_HALO];
+                uint64_t const tile_x0 = tile_id * PD_TILE_POS;
+
+                // (1) this thread's word: the valid positions m, their per-warp bucket counts (reductions without return value)
+                uint32_t const wi = threadIdx.x;
+                uint64_t const w0 = tw[wi], w1 = tw[wi + 1];
+                uint32_t m = clip_mask(tile_x0 + (uint64_t)wi * 32, P.x_begin, P.x_end);
+                if ( filter )
+                {
+                        #pragma unroll
+                        for ( uint32_t j = 0; j < 32; ++j )
+                                if ( bucket_at(w0, w1, j, bsh, bmask) - P.own_b_lo >= P.own_b_cnt ) m &= ~(1u << j);
+                }
+                #pragma unroll
+                for ( uint32_t j = 0; j < 32; ++j )
+                        if ( (m >> j) & 1 )
+                                atomicAdd(&S.wcnt[wid][bucket_at(w0, w1, j, bsh, bmask)], 1u);
+                __syncthreads();
+                // (2) bucket b (thread b): totals -> staging layout, global run reservation, per-warp running slots.  The exclusive
+                // scan over the 256 bucket totals is a warp scan + one barrier
+                uint32_t bstart = 0, reserved = 0;
+                {
+                        uint32_t tot = 0;
+                        #pragma unroll
+                        for ( int w = 0; w < PD_THREADS / 32; ++w ) tot += S.wcnt[w][threadIdx.x];
+                        uint32_t const incl = warp_incl_scan(tot, lane);
+                        if ( lane == 31 ) S.wsum[wid] = incl;
+                        // the run's first record is needed at the copy-out only: the global atomic that reserves it stays in
+                        // flight while the tile is ranked -- its result must not be touched before
+                        if ( tot )
+                        {
+                                bstart = P.bucket_start[threadIdx.x];
+                                reserved = atomicAdd(P.bucket_cursor + threadIdx.x * SC_CURSOR_STRIDE, tot);
+                        }
+                        __syncthreads();
+                        uint32_t base = 0;
+                        #pragma unroll
+                        for ( int w = 0; w < SC_MAX_BUCKETS / 32 - 1; ++w )
+                                if ( w < wid ) base += S.wsum[w];
+                        uint32_t const ex = base + incl - tot;
+                        S.loc[threadIdx.x] = ex;
+                        if ( threadIdx.x == SC_MAX_BUCKETS - 1 ) S.loc[SC_MAX_BUCKETS] = ex + tot;
+                        uint32_t run = ex;
+                        #pragma unroll
+                        for ( int w = 0; w < PD_THREADS / 32; ++w )
+                        {
+                                uint32_t const c = S.wcnt[w][threadIdx.x];
+                                S.wcnt[w][threadIdx.x] = run;
+                                run += c;
+                        }
+                }
+                __syncthreads();
+                // (3) warp multisplit: one position per lane and step; the group leader advances the warp's slot counter.
+                // The matches of four steps are issued together: their result latency is what this phase waits for
+                #pragma unroll
+                for ( uint32_t jb = 0; jb < 32; jb += 4 )
+                {
+                        uint32_t b[4], peers[4];
+                        #pragma unroll
+                        for ( uint32_t u = 0; u < 4; ++u )
+                        {
+                                b[u] = bucket_at(w0, w1, jb + u, bsh, bmask);
+                                peers[u] = peers_u8(b[u], (m >> (jb + u)) & 1);
+                        }
+                        #pragma unroll
+                        for ( uint32_t u = 0; u < 4; ++u )
+                        {
+                                bool const ok = (m >> (jb + u)) & 1;
+                                uint32_t const below = __popc(peers[u] & lt);
+                                uint32_t pre = 0;
+                                if ( ok ) pre = S.wcnt[wid][b[u]];
+                                __syncwarp();
+                                if ( ok && below == 0 ) S.wcnt[wid][b[u]] = pre + __popc(peers[u]);
+                                __syncwarp();
+                                if ( ok ) S.stage[pre + below] = (uint16_t)(wi * 32 + jb + u);
+                        }
+                }
+                // where staging slot 0 would go if it belonged to this bucket: the copy-out adds the slot number
+                S.dst[threadIdx.x] = S.area[threadIdx.x] + ((int64_t)(bstart + reserved) - (int64_t)S.loc[threadIdx.x]);
+                __syncthreads();
+                // the per-warp counters are free from here on (the copy-out does not read them): cleared for the next tile now,
+                // under the barrier that ends the copy-out
+                #pragma unroll
+                for ( int w = 0; w < PD_THREADS / 32; ++w ) S.wcnt[w][threadIdx.x] = 0;
+                // (4) copy out: consecutive threads write consecutive records of a bucket run; four records in flight per thread.
+                // A record is rebuilt from the three tile words around its offset; its bucket comes from its window
+                {
+                        uint32_t const n = S.loc[SC_MAX_BUCKETS];
+                        uint32_t const pos0 = (uint32_t)(tile_x0 - P.pos_base);     // may wrap for the clipped first tile; the sums below do not
+                        uint32_t i = threadIdx.x;
+                        for ( ; i < n; i += 4 * PD_THREADS )
+                        {
+                                uint32_t o[4];
+                                uint64_t wm[4], wa[4], wb[4];
+                                #pragma unroll
+                                for ( int u = 0; u < 4; ++u ) o[u] = i + u * PD_THREADS < n ? S.stage[i + u * PD_THREADS] : 0u;
+                                #pragma unroll
+                                for ( int u = 0; u < 4; ++u )
+                                {
+                                        uint32_t const k = o[u] >> 5;
+                                        wm[u] = tw[(int)k - 1]; wa[u] = tw[k]; wb[u] = tw[k + 1];
+                                }
+                                #pragma unroll
+                                for ( int u = 0; u < 4; ++u )
+                                {
+                                        if ( i + u * PD_THREADS >= n ) break;
+                                        uint32_t const j = o[u] & 31;
+                                        uint64_t const v = j ? ((wa[u] << (2*j)) | (wb[u] >> (64 - 2*j))) : wa[u];
+                                        uint32_t const before = (uint32_t)(j ? ((wm[u] << (2*j)) | (wa[u] >> (64 - 2*j))) : wm[u]);   // the 16 bases in front of the window
+                                        uint64_t const win = v >> fsh;
+                                        uint4 * const d = S.dst[((uint32_t)(v >> 32) >> bsh) & bmask];
+                                        d[i + u * PD_THREADS] = make_uint4((uint32_t)win, (uint32_t)(win >> 32), before, pos0 + o[u]);
+                                }
+                        }
+                }
+                __syncthreads();   // tile[buf], staging and the counters are free again
+        }
+}
+
+// ---- partition of a bucket shard -------------------------------------------------------------------
+// The multi-GPU form of the partition when the tables are sharded by bucket and every GPU holds the whole text
+// (real_gpu_set_bucket_shard): the rank reads EVERY position of the chunk but keeps only those whose bucket belongs
+// to it, 1/nranks of them.  Testing a position costs about one instruction (kept_positions: bit sliced over the 32
+// positions of a text word); ranking and staging a record is what is expensive.  So one light pass (k_own_list) writes
+// the kept positions as a dense list of 4-byte descriptors and counts them per bucket on the way -- no separate
+// histogram pass -- and a staged scatter kernel then forms the records of the list (k_part_scatter_list) at its usual cost
+// per record.  No record crosses NVLink: the only exchange of a bucket-sharded scan is the fold of the per-read results.
+//
+// The list kernel stages whole records: its positions are scattered over the text, so there is no tile of text words in
+// shared memory a record could be rebuilt from.  Tiles of 2048 listed positions.
+static const int PS_THREADS = 256;                            // threads per CTA; thread b also acts for bucket b
+static const int PS_PPT = 8;                                  // listed positions per thread
+static const int PS_TILE_POS = PS_THREADS * PS_PPT;           // 2048
+
+struct ListScatterSmem
+{
+        uint4 stage[PS_TILE_POS];                          // record, bucket-major
+        uint32_t wcnt[PS_THREADS / 32][SC_MAX_BUCKETS];    // per-warp counts, then running slots
+        uint32_t loc[SC_MAX_BUCKETS + 1];                  // first staging slot of a bucket
+        uint32_t wsum[SC_MAX_BUCKETS / 32];                // bucket totals per warp of bucket threads (exclusive scan)
+        uint4 * dst[SC_MAX_BUCKETS];                       // per tile: record area + first record of the tile's run - first staging slot
+};
+
+__global__ void __launch_bounds__(PS_THREADS, 1024 / PS_THREADS) k_part_scatter_list(ScanParams P)
+{
+        extern __shared__ __align__(128) unsigned char sc_smem[];
+        ListScatterSmem & S = *reinterpret_cast<ListScatterSmem *>(sc_smem);
+
+        uint64_t const nlist = *P.list_count;
+        uint64_t const end_tile = (nlist + PS_TILE_POS - 1) / PS_TILE_POS;
         uint32_t const bbits = P.bucket_bits;
         uint32_t const bsh = 64 - (bbits ? bbits : 1);
         uint32_t const bmask = bbits ? 0xFFFFFFFFu : 0u;
@@ -430,40 +628,18 @@ __global__ void __launch_bounds__(PS_THREADS, 1024 / PS_THREADS) k_part_scatter(
         int const lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
         uint32_t const lt = (1u << lane) - 1;
 
-        if ( ! LIST && threadIdx.x == 0 )
-        {
-                mbar_init(&S.bar[0], 1);
-                mbar_init(&S.bar[1], 1);
-                asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        }
-        bool const bt = threadIdx.x < (uint32_t)SC_MAX_BUCKETS;       // this thread also acts for bucket threadIdx.x
-        if ( bt )
-        {
-                #pragma unroll
-                for ( int w = 0; w < PS_THREADS / 32; ++w ) S.wcnt[w][threadIdx.x] = 0;
-                S.area[threadIdx.x] = P.peer_recs[bucket_owner(P, threadIdx.x)];
-        }
+        #pragma unroll
+        for ( int w = 0; w < PS_THREADS / 32; ++w ) S.wcnt[w][threadIdx.x] = 0;
         __syncthreads();
 
-        uint64_t tile_id = first_tile + blockIdx.x;
-        if ( ! LIST && threadIdx.x == 0 && tile_id < end_tile )
-        {
-                mbar_expect_tx(&S.bar[0], PS_SMEM_WORDS * 8);
-                bulk_load(&S.tile[0][0], P.text + (int64_t)tile_id * PS_TILE_WORDS - SC_HALO, PS_SMEM_WORDS * 8, &S.bar[0]);
-        }
-
-        for ( uint32_t it = 0; tile_id < end_tile; tile_id += gridDim.x, ++it )
+        for ( uint64_t tile_id = blockIdx.x; tile_id < end_tile; tile_id += gridDim.x )
         {
                 // the PS_PPT positions of this thread: window word v, the 32 bases in front of it, position field, validity mask m
                 uint64_t wv[PS_PPT];
                 uint32_t wbefore[PS_PPT], wpos[PS_PPT];
-                uint32_t m;
-                uint32_t pos0;
-                if constexpr ( LIST )
+                uint32_t m = 0;
                 {
                         uint64_t const i0 = tile_id * PS_TILE_POS + (uint64_t)threadIdx.x * PS_PPT;
-                        m = 0;
-                        pos0 = 0;
                         #pragma unroll
                         for ( uint32_t u = 0; u < PS_PPT; ++u )
                         {
@@ -479,37 +655,6 @@ __global__ void __launch_bounds__(PS_THREADS, 1024 / PS_THREADS) k_part_scatter(
                                 m |= (ok ? 1u : 0u) << u;
                         }
                 }
-                else
-                {
-                        uint32_t const buf = it & 1;
-                        uint64_t const next_tile = tile_id + gridDim.x;
-                        if ( threadIdx.x == 0 && next_tile < end_tile )
-                        {
-                                mbar_expect_tx(&S.bar[buf ^ 1], PS_SMEM_WORDS * 8);
-                                bulk_load(&S.tile[buf ^ 1][0], P.text + (int64_t)next_tile * PS_TILE_WORDS - SC_HALO, PS_SMEM_WORDS * 8, &S.bar[buf ^ 1]);
-                        }
-                        mbar_wait(&S.bar[buf], (it >> 1) & 1);
-                        uint64_t const tile_x0 = tile_id * PS_TILE_POS;
-                        uint32_t const wi = threadIdx.x / PS_TPW, j0 = (threadIdx.x % PS_TPW) * PS_PPT;
-                        uint64_t const wm = S.tile[buf][SC_HALO + wi - 1], w0 = S.tile[buf][SC_HALO + wi], w1 = S.tile[buf][SC_HALO + wi + 1];
-                        m = (clip_mask(tile_x0 + (uint64_t)wi * 32, P.x_begin, P.x_end) >> j0) & (uint32_t)((1ull << PS_PPT) - 1);
-                        if ( PS_PPT == 8 && P.own_b_cnt < SC_MAX_BUCKETS )
-                        {
-                                // bucket shard with many own buckets (two ranks): every position is looked at here, only the own ones
-                                // are ranked and staged (with few own buckets the list form above is cheaper)
-                                uint32_t top;
-                                m &= own_mask8(w0, w1, j0, P.own_b_lo, P.own_b_cnt, top);
-                        }
-                        pos0 = (uint32_t)(tile_x0 - P.pos_base);     // may wrap for the clipped first tile; the sums below do not
-                        #pragma unroll
-                        for ( uint32_t u = 0; u < PS_PPT; ++u )
-                        {
-                                uint32_t const j = j0 + u;
-                                wv[u] = j ? ((w0 << (2*j)) | (w1 >> (64 - 2*j))) : w0;
-                                wbefore[u] = (uint32_t)(j ? ((wm << (2*j)) | (w0 >> (64 - 2*j))) : wm);       // the 16 bases that end in front of the window
-                                wpos[u] = wi * 32 + j;
-                        }
-                }
 
                 // (1) per-warp bucket counts (reductions without return value)
                 #pragma unroll
@@ -517,50 +662,38 @@ __global__ void __launch_bounds__(PS_THREADS, 1024 / PS_THREADS) k_part_scatter(
                         if ( (m >> u) & 1 )
                                 atomicAdd(&S.wcnt[wid][(uint32_t)(wv[u] >> bsh) & bmask], 1u);
                 __syncthreads();
-                // (2) bucket b (thread b): totals -> staging layout, global run reservation, per-warp running slots.  The exclusive
-                // scan over the 256 bucket totals is a warp scan + one barrier (the generic block scan has three, and the block
-                // barriers are a fifth of this kernel's stall samples)
-                uint32_t bstart = 0, reserved = 0;       // basev = bstart + reserved, summed only where it is needed (see below)
+                // (2) bucket b (thread b): totals -> staging layout, global run reservation, per-warp running slots
+                uint32_t bstart = 0, reserved = 0;
                 {
                         uint32_t tot = 0;
-                        if ( bt )
-                        {
-                                #pragma unroll
-                                for ( int w = 0; w < PS_THREADS / 32; ++w ) tot += S.wcnt[w][threadIdx.x];
-                        }
+                        #pragma unroll
+                        for ( int w = 0; w < PS_THREADS / 32; ++w ) tot += S.wcnt[w][threadIdx.x];
                         uint32_t const incl = warp_incl_scan(tot, lane);
-                        if ( bt && lane == 31 ) S.wsum[wid] = incl;
-                        // the run's first record is needed at the copy-out only: the global atomic that reserves it stays in
-                        // flight while the tile is ranked -- its result must not be touched before (an addition right here
-                        // made every thread wait for the round trip: 12 % of the kernel's stall samples)
+                        if ( lane == 31 ) S.wsum[wid] = incl;
                         if ( tot )
                         {
                                 bstart = P.bucket_start[threadIdx.x];
                                 reserved = atomicAdd(P.bucket_cursor + threadIdx.x * SC_CURSOR_STRIDE, tot);
                         }
                         __syncthreads();
-                        if ( bt )
+                        uint32_t base = 0;
+                        #pragma unroll
+                        for ( int w = 0; w < SC_MAX_BUCKETS / 32 - 1; ++w )
+                                if ( w < wid ) base += S.wsum[w];
+                        uint32_t const ex = base + incl - tot;
+                        S.loc[threadIdx.x] = ex;
+                        if ( threadIdx.x == SC_MAX_BUCKETS - 1 ) S.loc[SC_MAX_BUCKETS] = ex + tot;
+                        uint32_t run = ex;
+                        #pragma unroll
+                        for ( int w = 0; w < PS_THREADS / 32; ++w )
                         {
-                                uint32_t base = 0;
-                                #pragma unroll
-                                for ( int w = 0; w < SC_MAX_BUCKETS / 32 - 1; ++w )
-                                        if ( w < wid ) base += S.wsum[w];
-                                uint32_t const ex = base + incl - tot;
-                                S.loc[threadIdx.x] = ex;
-                                if ( threadIdx.x == SC_MAX_BUCKETS - 1 ) S.loc[SC_MAX_BUCKETS] = ex + tot;
-                                uint32_t run = ex;
-                                #pragma unroll
-                                for ( int w = 0; w < PS_THREADS / 32; ++w )
-                                {
-                                        uint32_t const c = S.wcnt[w][threadIdx.x];
-                                        S.wcnt[w][threadIdx.x] = run;
-                                        run += c;
-                                }
+                                uint32_t const c = S.wcnt[w][threadIdx.x];
+                                S.wcnt[w][threadIdx.x] = run;
+                                run += c;
                         }
                 }
                 __syncthreads();
-                // (3) warp multisplit: one position per lane and step; the group leader advances the warp's slot counter.
-                // The matches of four steps are issued together: their result latency is what this phase waits for.
+                // (3) warp multisplit: one position per lane and step; the group leader advances the warp's slot counter
                 #pragma unroll
                 for ( uint32_t jb = 0; jb < PS_PPT; jb += 4 )
                 {
@@ -583,25 +716,16 @@ __global__ void __launch_bounds__(PS_THREADS, 1024 / PS_THREADS) k_part_scatter(
                                 __syncwarp();
                                 if ( ok )
                                 {
-                                        uint32_t const slot = pre + below;
                                         uint64_t const win = wv[jb + u] >> fsh;
-                                        S.stage[slot] = make_uint4((uint32_t)win, (uint32_t)(win >> 32), wbefore[jb + u], wpos[jb + u] + pos0);
+                                        S.stage[pre + below] = make_uint4((uint32_t)win, (uint32_t)(win >> 32), wbefore[jb + u], wpos[jb + u]);
                                 }
                         }
                 }
-                // where staging slot 0 would go if it belonged to this bucket: the copy-out adds the slot number
-                if ( bt ) S.dst[threadIdx.x] = S.area[threadIdx.x] + ((int64_t)(bstart + reserved) - (int64_t)S.loc[threadIdx.x]);
+                S.dst[threadIdx.x] = P.recs + ((int64_t)(bstart + reserved) - (int64_t)S.loc[threadIdx.x]);
                 __syncthreads();
-                // the per-warp counters are free from here on (the copy-out does not read them): cleared for the next tile now,
-                // under the barrier that ends the copy-out
-                if ( bt )
-                {
-                        #pragma unroll
-                        for ( int w = 0; w < PS_THREADS / 32; ++w ) S.wcnt[w][threadIdx.x] = 0;
-                }
-                // (4) copy out: consecutive threads write consecutive records of a bucket run; four records in flight per thread.
-                // The bucket of a record is recomputed from its window (three ALU instructions) instead of being staged beside it:
-                // the kernel is limited by its shared-memory instructions, not by arithmetic
+                #pragma unroll
+                for ( int w = 0; w < PS_THREADS / 32; ++w ) S.wcnt[w][threadIdx.x] = 0;
+                // (4) copy out: consecutive threads write consecutive records of a bucket run; four records in flight per thread
                 {
                         uint32_t const n = S.loc[SC_MAX_BUCKETS];
                         uint32_t i = threadIdx.x;
@@ -621,18 +745,10 @@ __global__ void __launch_bounds__(PS_THREADS, 1024 / PS_THREADS) k_part_scatter(
                                 S.dst[(uint32_t)(((((uint64_t)r.y << 32) | r.x) << fsh) >> bsh) & bmask][i] = r;
                         }
                 }
-                __syncthreads();   // tile[buf], staging and the counters are free again
+                __syncthreads();   // staging and the counters are free again
         }
 }
 
-// ---- partition of a bucket shard -------------------------------------------------------------------
-// The multi-GPU form of the partition when the tables are sharded by bucket and every GPU holds the whole text
-// (real_gpu_set_bucket_shard): the rank reads EVERY position of the chunk but keeps only those whose bucket belongs
-// to it, 1/nranks of them.  Testing a position costs about one instruction (kept_positions: bit sliced over the 32
-// positions of a text word); ranking and staging a record is what is expensive.  So one light pass (k_own_list) writes
-// the kept positions as a dense list of 4-byte descriptors and counts them per bucket on the way -- no separate
-// histogram pass -- and the staged scatter kernel then runs on the list (k_part_scatter<true>) at its usual cost per
-// record.  No record crosses NVLink: the only exchange of a bucket-sharded scan is the fold of the per-read results.
 static const int OL_THREADS = 256;
 static const int OL_WPT = 4;                                  // consecutive text words per thread and tile
 static const int OL_TILE_WORDS = OL_THREADS * OL_WPT;
