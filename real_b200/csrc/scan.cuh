@@ -390,8 +390,8 @@ __global__ void __launch_bounds__(SC_THREADS) k_part_hist(ScanParams P)
 // Records are first laid out bucket by bucket in shared memory and then copied out run by run, so every global store
 // instruction writes whole consecutive records of one bucket: scattering records straight from the threads that produce
 // them leaves ~200 KB of half-written lines open per CTA, more than L2 holds for a full grid (measured: 2 GB of DRAM reads
-// and 5 GB of writes for 3 GB of records, 10 ms per 250 M positions).  Ranks come from a warp-level multisplit (peers_u8
-// on the bucket id: one ballot per bit): shared-memory atomics that return a value serialise far too much for this.
+// and 5 GB of writes for 3 GB of records, 10 ms per 250 M positions).  Ranks come from a warp-level multisplit (ballots
+// of the bucket bits: rank_word): shared-memory atomics that return a value serialise far too much for this.
 //
 // Dense form (every position of the chunk, or those of the own buckets of a two-rank bucket shard): tiles of 8192
 // positions, one text word per thread.  What is staged is the 2-byte offset of a position in its tile, not its 16-byte
@@ -412,6 +412,7 @@ struct ScatterSmem
 {
         uint64_t tile[2][PD_SMEM_WORDS];                   // bulk-copy destinations first: 16-byte aligned
         uint64_t bar[2];
+        uint4 quad[2 * PD_TILE_WORDS];                     // quad h: the 64 bases [16h-16, 16h+48) of the tile, as 4 half-words
         uint4 * dst[SC_MAX_BUCKETS];                       // per tile: record area of the bucket's owner + first record of the tile's run - first staging slot
         uint4 * area[SC_MAX_BUCKETS];                      // record area of the bucket's owner
         uint32_t wcnt[PD_THREADS / 32][SC_MAX_BUCKETS];    // per-warp counts, then running slots
@@ -426,6 +427,60 @@ __device__ __forceinline__ uint32_t bucket_at(uint64_t w0, uint64_t w1, uint32_t
         uint32_t const top = j < 16 ? __funnelshift_l((uint32_t)w0, (uint32_t)(w0 >> 32), 2 * j)
                                     : __funnelshift_l((uint32_t)(w1 >> 32), (uint32_t)w0, 2 * j - 32);
         return (top >> bsh) & bmask;
+}
+
+// "the lanes whose bit p of the stream w0:w1 (p = 0: the top bit of w0) equals mine", one ballot per bit plane
+__device__ __forceinline__ uint32_t agree_plane(uint64_t w0, uint64_t w1, uint32_t p)
+{
+        uint32_t const half = p < 32 ? (uint32_t)(w0 >> 32) : p < 64 ? (uint32_t)w0 : (uint32_t)(w1 >> 32);
+        uint32_t bal, flip;
+        ballot_bit(half, 0x80000000u >> (p & 31), bal, flip);
+        return bal ^ flip;
+}
+
+// Phase 3 of k_part_scatter: ranks the valid positions m of the thread's text word w0 (w1 = the word behind it) inside
+// their buckets with a warp multisplit and stages their tile offsets.  The matches of four steps are issued together:
+// their result latency is what this phase waits for.  PLANES (8-bit buckets): the bucket of position j is bits 2j ..
+// 2j+7 of the stream w0:w1, so consecutive positions share six of their eight bit planes; each plane's ballot is taken
+// once for the word (70 ballots for its 32 positions, against 256 for one multisplit per position).
+template <bool PLANES>
+__device__ __forceinline__ void rank_word(ScatterSmem & S, uint64_t w0, uint64_t w1, uint32_t m, uint32_t wi, int wid, uint32_t lt,
+                                          uint32_t bsh, uint32_t bmask)
+{
+        uint32_t E[72];
+        #pragma unroll
+        for ( uint32_t jb = 0; jb < 32; jb += 4 )
+        {
+                if ( PLANES )
+                {
+                        #pragma unroll
+                        for ( uint32_t p = jb ? 2 * jb + 6 : 0; p < 2 * jb + 14; ++p ) E[p] = agree_plane(w0, w1, p);
+                }
+                uint32_t b[4], peers[4];
+                #pragma unroll
+                for ( uint32_t u = 0; u < 4; ++u )
+                {
+                        uint32_t const j = jb + u;
+                        b[u] = bucket_at(w0, w1, j, bsh, bmask);
+                        if ( PLANES )
+                                peers[u] = __ballot_sync(0xffffffffu, (m >> j) & 1) & E[2*j] & E[2*j+1] & E[2*j+2] & E[2*j+3]
+                                           & E[2*j+4] & E[2*j+5] & E[2*j+6] & E[2*j+7];
+                        else
+                                peers[u] = peers_u8(b[u], (m >> j) & 1);
+                }
+                #pragma unroll
+                for ( uint32_t u = 0; u < 4; ++u )
+                {
+                        bool const ok = (m >> (jb + u)) & 1;
+                        uint32_t const below = __popc(peers[u] & lt);
+                        uint32_t pre = 0;
+                        if ( ok ) pre = S.wcnt[wid][b[u]];
+                        __syncwarp();
+                        if ( ok && below == 0 ) S.wcnt[wid][b[u]] = pre + __popc(peers[u]);
+                        __syncwarp();
+                        if ( ok ) S.stage[pre + below] = (uint16_t)(wi * 32 + jb + u);
+                }
+        }
 }
 
 __global__ void __launch_bounds__(PD_THREADS, PD_MINB) k_part_scatter(ScanParams P)
@@ -474,9 +529,16 @@ __global__ void __launch_bounds__(PD_THREADS, PD_MINB) k_part_scatter(ScanParams
                 const uint64_t * tw = &S.tile[buf][SC_HALO];
                 uint64_t const tile_x0 = tile_id * PD_TILE_POS;
 
-                // (1) this thread's word: the valid positions m, their per-warp bucket counts (reductions without return value)
+                // (1) this thread's word: the two quads of its half-words for the copy-out (the halo covers tw[-1] and
+                // tw[PD_TILE_WORDS]), the valid positions m, their per-warp bucket counts (reductions without return value)
                 uint32_t const wi = threadIdx.x;
                 uint64_t const w0 = tw[wi], w1 = tw[wi + 1];
+                {
+                        uint32_t const wm_lo = (uint32_t)tw[(int)wi - 1];
+                        uint32_t const w0_hi = (uint32_t)(w0 >> 32), w0_lo = (uint32_t)w0, w1_hi = (uint32_t)(w1 >> 32);
+                        S.quad[2 * wi] = make_uint4(wm_lo, w0_hi, w0_lo, w1_hi);
+                        S.quad[2 * wi + 1] = make_uint4(w0_hi, w0_lo, w1_hi, (uint32_t)w1);
+                }
                 uint32_t m = clip_mask(tile_x0 + (uint64_t)wi * 32, P.x_begin, P.x_end);
                 if ( filter )
                 {
@@ -523,31 +585,9 @@ __global__ void __launch_bounds__(PD_THREADS, PD_MINB) k_part_scatter(ScanParams
                         }
                 }
                 __syncthreads();
-                // (3) warp multisplit: one position per lane and step; the group leader advances the warp's slot counter.
-                // The matches of four steps are issued together: their result latency is what this phase waits for
-                #pragma unroll
-                for ( uint32_t jb = 0; jb < 32; jb += 4 )
-                {
-                        uint32_t b[4], peers[4];
-                        #pragma unroll
-                        for ( uint32_t u = 0; u < 4; ++u )
-                        {
-                                b[u] = bucket_at(w0, w1, jb + u, bsh, bmask);
-                                peers[u] = peers_u8(b[u], (m >> (jb + u)) & 1);
-                        }
-                        #pragma unroll
-                        for ( uint32_t u = 0; u < 4; ++u )
-                        {
-                                bool const ok = (m >> (jb + u)) & 1;
-                                uint32_t const below = __popc(peers[u] & lt);
-                                uint32_t pre = 0;
-                                if ( ok ) pre = S.wcnt[wid][b[u]];
-                                __syncwarp();
-                                if ( ok && below == 0 ) S.wcnt[wid][b[u]] = pre + __popc(peers[u]);
-                                __syncwarp();
-                                if ( ok ) S.stage[pre + below] = (uint16_t)(wi * 32 + jb + u);
-                        }
-                }
+                // (3) warp multisplit: one position per lane and step; the group leader advances the warp's slot counter
+                if ( bbits == 8 ) rank_word<true>(S, w0, w1, m, wi, wid, lt, bsh, bmask);
+                else rank_word<false>(S, w0, w1, m, wi, wid, lt, bsh, bmask);
                 // where staging slot 0 would go if it belonged to this bucket: the copy-out adds the slot number
                 S.dst[threadIdx.x] = S.area[threadIdx.x] + ((int64_t)(bstart + reserved) - (int64_t)S.loc[threadIdx.x]);
                 __syncthreads();
@@ -556,7 +596,8 @@ __global__ void __launch_bounds__(PD_THREADS, PD_MINB) k_part_scatter(ScanParams
                 #pragma unroll
                 for ( int w = 0; w < PD_THREADS / 32; ++w ) S.wcnt[w][threadIdx.x] = 0;
                 // (4) copy out: consecutive threads write consecutive records of a bucket run; four records in flight per thread.
-                // A record is rebuilt from the three tile words around its offset; its bucket comes from its window
+                // A record at offset o = 16h + r needs the bases [o-16, o+32), which lie in quad h: one 16-byte load, then
+                // funnel shifts by 2r cut the 16 bases in front and the two halves of the window.  Its bucket comes from its window
                 {
                         uint32_t const n = S.loc[SC_MAX_BUCKETS];
                         uint32_t const pos0 = (uint32_t)(tile_x0 - P.pos_base);     // may wrap for the clipped first tile; the sums below do not
@@ -564,29 +605,26 @@ __global__ void __launch_bounds__(PD_THREADS, PD_MINB) k_part_scatter(ScanParams
                         for ( ; i < n; i += 4 * PD_THREADS )
                         {
                                 uint32_t o[4];
-                                uint64_t wm[4], wa[4], wb[4];
+                                uint4 q[4];
                                 #pragma unroll
                                 for ( int u = 0; u < 4; ++u ) o[u] = i + u * PD_THREADS < n ? S.stage[i + u * PD_THREADS] : 0u;
                                 #pragma unroll
-                                for ( int u = 0; u < 4; ++u )
-                                {
-                                        uint32_t const k = o[u] >> 5;
-                                        wm[u] = tw[(int)k - 1]; wa[u] = tw[k]; wb[u] = tw[k + 1];
-                                }
+                                for ( int u = 0; u < 4; ++u ) q[u] = S.quad[o[u] >> 4];
                                 #pragma unroll
                                 for ( int u = 0; u < 4; ++u )
                                 {
                                         if ( i + u * PD_THREADS >= n ) break;
-                                        uint32_t const j = o[u] & 31;
-                                        uint64_t const v = j ? ((wa[u] << (2*j)) | (wb[u] >> (64 - 2*j))) : wa[u];
-                                        uint32_t const before = (uint32_t)(j ? ((wm[u] << (2*j)) | (wa[u] >> (64 - 2*j))) : wm[u]);   // the 16 bases in front of the window
-                                        uint64_t const win = v >> fsh;
-                                        uint4 * const d = S.dst[((uint32_t)(v >> 32) >> bsh) & bmask];
+                                        uint32_t const sh = 2 * (o[u] & 15);
+                                        uint32_t const before = __funnelshift_l(q[u].y, q[u].x, sh);   // the 16 bases in front of the window
+                                        uint32_t const vhi = __funnelshift_l(q[u].z, q[u].y, sh);
+                                        uint32_t const vlo = __funnelshift_l(q[u].w, q[u].z, sh);
+                                        uint64_t const win = (((uint64_t)vhi << 32) | vlo) >> fsh;
+                                        uint4 * const d = S.dst[(vhi >> bsh) & bmask];
                                         d[i + u * PD_THREADS] = make_uint4((uint32_t)win, (uint32_t)(win >> 32), before, pos0 + o[u]);
                                 }
                         }
                 }
-                __syncthreads();   // tile[buf], staging and the counters are free again
+                __syncthreads();   // tile[buf], the quads, staging and the counters are free again
         }
 }
 
